@@ -8,16 +8,19 @@ One "step" = encode the whole batch (RGB -> channel payloads + offset table) and
 with inputs already resident in HBM; `e2e` is the same metric through the host-buffer C-ABI calls
 (hoh_encode_images_s0_host / hoh_decode_images_s0_host) with H2D/D2H inside the timed region.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 N > 1: launched by torchrun, one rank per GPU, images sharded by index, no data-path collective.
 """
 import argparse
+import atexit
 import ctypes as C
 import importlib.util
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -41,11 +44,18 @@ def _load(name, path):
 # ------------------------------------------------------------------------------------------------
 # synthetic inputs (tools/synth_gen.c, SURVEY section 8(d))
 # ------------------------------------------------------------------------------------------------
+_SYNTH_DIR = None
+
+
 def synth_lib():
-    so = os.path.join(ROOT, "tools", "libsynth.so")
-    src = os.path.join(ROOT, "tools", "synth_gen.c")
-    if not os.path.exists(so) or os.path.getmtime(src) > os.path.getmtime(so):
-        subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-o", so, src])
+    """tools/synth_gen.c compiled into a per-process temporary directory: the tree may be read-only."""
+    global _SYNTH_DIR
+    if _SYNTH_DIR is None:
+        _SYNTH_DIR = tempfile.mkdtemp(prefix="hoh_bench_")
+        atexit.register(shutil.rmtree, _SYNTH_DIR, True)
+    so = os.path.join(_SYNTH_DIR, "libsynth.so")
+    if not os.path.exists(so):
+        subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-o", so, os.path.join(ROOT, "tools", "synth_gen.c")])
     L = C.CDLL(so)
     L.synth_rgb_batch.restype = None
     L.synth_rgb_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_uint64, C.c_size_t]
@@ -105,7 +115,7 @@ class ClockSampler:
             self.thread.start()
         except Exception:
             self.nvml = None
-            self.path = f"/tmp/hoh_clocks_{os.getpid()}.csv"
+            self.path = os.path.join(tempfile.gettempdir(), f"hoh_clocks_{os.getpid()}.csv")
             try:
                 self.out = open(self.path, "w")
                 self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.idx), f"--query-gpu={self.Q}",
@@ -250,7 +260,7 @@ def cpu_whole_tool(images, w, h, mode, cores, seed0=1):
     """BASELINE.md section 3.1: stock choh, one process per core, over `images` images.  MB/s of raw RGB over the
     busy time of the slowest worker.  Encode only: the reference's dhoh cannot decode choh's output."""
     import multiprocessing as mp
-    import tempfile
+    synth_lib()  # compiled once, before the workers fork
     per = [images // cores + (1 if i < images % cores else 0) for i in range(cores)]
     with tempfile.TemporaryDirectory() as tmp:
         jobs, seed = [], seed0
@@ -370,6 +380,7 @@ def cpu_hot_path(sample_images, w, h, cores, seed0=1):
     """Times the reference CPU hot path (encode + decode, LZ excluded: NUKE == 0) on `cores`
     processes over `sample_images` images.  Returns dict(value MB/s, t_enc, t_dec, kind)."""
     import multiprocessing as mp
+    synth_lib()  # compiled once, before the workers fork
     per = [sample_images // cores + (1 if i < sample_images % cores else 0) for i in range(cores)]
     jobs, seed = [], seed0
     for n in per:
@@ -586,7 +597,10 @@ def run_config_tiles(g, mod, shard, rank, world, host_threads, hbm_peak, barrier
             return tb - ta, time.perf_counter() - tb
         e2e_once()
         barrier()
-        te, td = e2e_once()
+        te = td = 0.0
+        for _ in range(steps):
+            a, b = e2e_once()
+            te, td = te + a / steps, td + b / steps
         e2e = {"encode_ms": 1e3 * te, "decode_ms": 1e3 * td,
                "ok": bool((rec["status"] == 0).all() and (st == 0).all() and np.array_equal(back, src)),
                "h2d": raw + int(off[-1]), "d2h": raw + int(off[-1])}
@@ -691,6 +705,44 @@ def run_config_static(g, mod, shard, rank, world, hbm_peak, barrier, log2n, step
             "roundtrip_exact_and_oracle_parity": all_ok}
 
 
+DUMP_IMAGES = 4  # images whose payload bytes and decoded RGB are written: ~20 MB as float32
+DUMP_STREAMS = 1 << 18  # per-stream records written at most: 9 float64 each, ~19 MB
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, mod, geom, n_img, d_res, d_packed, d_off, d_back, d_st):
+    """What a caller of hoh_encode_images_s0 + hoh_decode_images_s0 receives after the last timed step, so that two
+    builds can be compared file by file: per-stream records (payload start / end, encode result fields, decode
+    status) as float64 for every stream, or for a fixed, seeded sample of DUMP_STREAMS of them, and the payload
+    bytes and decoded RGB of a fixed, seeded sample of DUMP_IMAGES images as float32 (the batch is gigabytes)."""
+    spi = geom.streams_per_image
+    n_streams = n_img * spi
+    off = d_off.download(np.uint64, n_streams + 1)
+    res = d_res.download(mod.RESULT_DT, n_streams)
+    keep = np.arange(n_streams)
+    if n_streams > DUMP_STREAMS:
+        keep = np.sort(np.random.default_rng(1).choice(n_streams, DUMP_STREAMS, replace=False))
+    arrays = {"streams": keep, "stream_start": off[keep], "stream_end": off[keep + 1],
+              "decode_status": d_st.download(np.int32, n_streams)[keep]}
+    for f in mod.RESULT_DT.names:
+        arrays[f"encode_{f}"] = res[f][keep]
+    arrays = {k: a.astype(np.float64) for k, a in arrays.items()}
+    pick = np.sort(np.random.default_rng(0).choice(n_img, min(DUMP_IMAGES, n_img), replace=False))
+    payload, rgb = [], []
+    for i in pick:
+        lo, hi = int(off[i * spi]), int(off[(i + 1) * spi])
+        payload.append(d_packed.download(np.uint8, hi - lo, offset=lo))
+        rgb.append(d_back.download(np.uint8, W * H * 3, offset=int(i) * W * H * 3).reshape(H, W, 3))
+    arrays["sample_images"] = pick.astype(np.float64)
+    arrays["sample_payload"] = np.concatenate(payload).astype(np.float32)
+    arrays["sample_decoded_rgb"] = np.stack(rgb).astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -707,7 +759,11 @@ def main():
     ap.add_argument("--frames", type=int, default=256, help="config 3: 3840x2160 frames in the whole job (strong scaling)")
     ap.add_argument("--thumbs", type=int, default=8192, help="config 5: 256x256 thumbnails per GPU")
     ap.add_argument("--static-log2", type=int, default=30, help="config 4: log2 of the symbols per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     extra = [int(x) for x in args.configs.split(",") if x.strip()]
 
     rank = int(os.environ.get("RANK", "0"))
@@ -827,6 +883,8 @@ def main():
     barrier()
     clk = clocks.stop()
     launches = g.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, mod, geom, n_img, d_res, d_packed, d_off, d_back, d_st)
 
     # per-kernel profile of one step (separate pass, CUDA events after every launch)
     g.profile_begin()
@@ -893,7 +951,7 @@ def main():
         barrier()
         g.timer_start(1)
         t0 = time.perf_counter()
-        e_steps = max(1, min(steps, 3))
+        e_steps = steps
         for _ in range(e_steps):
             total = e2e_step()
         g.timer_stop(1)
@@ -946,15 +1004,15 @@ def main():
             configs_out["config3"] = run_config_tiles(g, mod, shard, rank, world, host_threads, hbm_peak_all, barrier,
                                                       name="256 x 3840x2160 -s2, frames sharded across the GPUs (strong scaling)",
                                                       w=3840, h=2160, mode=2, total_images=args.frames, strong=True,
-                                                      parity_tiles=4, steps=3, e2e_leg=not args.no_e2e)
+                                                      parity_tiles=4, steps=steps, e2e_leg=not args.no_e2e)
         elif c == 5:
             configs_out["config5"] = run_config_tiles(g, mod, shard, rank, world, host_threads, hbm_peak_all, barrier,
                                                       name=f"slice of the 1M 256x256 thumbnails at -s4: {args.thumbs} per GPU "
                                                            f"(weak scaling; the full 10^6 / 8 GPUs = {125000 // args.thumbs + 1} such chunks per GPU)",
                                                       w=256, h=256, mode=4, total_images=args.thumbs, strong=False,
-                                                      parity_tiles=2, steps=5, e2e_leg=not args.no_e2e)
+                                                      parity_tiles=2, steps=steps, e2e_leg=not args.no_e2e)
         elif c == 4:
-            configs_out["config4"] = run_config_static(g, mod, shard, rank, world, hbm_peak_all, barrier, args.static_log2, steps=3)
+            configs_out["config4"] = run_config_static(g, mod, shard, rank, world, hbm_peak_all, barrier, args.static_log2, steps)
 
     total_ms = rmax(total_ms)
     t_enc, t_dec = rmax(t_enc), rmax(t_dec)

@@ -1,5 +1,5 @@
 """Pins the CPU oracle (oracle/hoh_oracle.c) to the real reference compiled from its own sources
-(oracle/_ref/libhohref.so).  CPU only.  Skipped when the reference library was never built."""
+(oracle/_ref/libhohref.so).  CPU only.  The comparisons skip when the reference library was never built."""
 import ctypes as C
 
 import numpy as np
@@ -7,7 +7,7 @@ import pytest
 
 import oracle_lib as ol
 
-pytestmark = pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref/libhohref.so not built")
+needs_ref = pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref/libhohref.so not built")
 
 STOCK = [0x0001, 0x0002, 0x0020, 0x0010, 0xffbf, 0x0003, 0xfffd, 0xfffb, 0xfff7, 0xffef, 0xffdf,
          0xff7f, 0xfdff, 0xffff]
@@ -31,6 +31,7 @@ def _symbols(rng, kind, n, rangev):
     return s.astype(np.uint16)
 
 
+@needs_ref
 def test_encode_entropy_random_streams():
     """entropy_encoding.hpp:8 — header, table modes 1/2, rANS payload, stored fallback, n = 0."""
     rng = np.random.default_rng(0)
@@ -51,6 +52,7 @@ def test_encode_entropy_random_streams():
     assert checked > 1000
 
 
+@needs_ref
 def test_decode_entropy_matches_reference_where_it_can_parse():
     """entropy_decoding.hpp:134 with reference semantics (flags=0), prob_bits <= 15 (D9)."""
     rng = np.random.default_rng(3)
@@ -83,6 +85,7 @@ def test_decode_roundtrip_all_prob_bits_fixed_mode():
         assert (d == sym).all() and bp == len(stream)
 
 
+@needs_ref
 def test_normalize_freqs():
     """stattools.hpp:13"""
     rng = np.random.default_rng(1)
@@ -128,6 +131,7 @@ def _plane(rng, w, h, depth, kind):
     return np.full(w * h, int(rng.integers(0, c)), np.uint16)
 
 
+@needs_ref
 def test_prediction_and_unprediction():
     """prediction.hpp:6/46/153, unprediction.hpp:6 incl. LZ back-references and clipped cells."""
     rng = np.random.default_rng(2)
@@ -169,6 +173,7 @@ def test_prediction_and_unprediction():
         assert (fu == p).all()
 
 
+@needs_ref
 def test_colour_transform():
     """channel.hpp:63-79 and its algebraic inverse."""
     rng = np.random.default_rng(5)
@@ -189,6 +194,7 @@ def test_colour_transform():
         assert (pa == pb).all()
 
 
+@needs_ref
 def test_layer_encode_all_modes():
     """layer_encode.hpp:11 byte-for-byte, modes 0-4, depth 8/9, with and without NUKE (D7 incl.)."""
     rng = np.random.default_rng(6)
@@ -207,6 +213,7 @@ def test_layer_encode_all_modes():
         assert a.tobytes() == b.tobytes(), (w, h, depth, mode)
 
 
+@needs_ref
 def test_static_table_rans():
     """rans64.hpp:262 (reciprocal form) == divide form, rans64.hpp:107-142 decode (config 4)."""
     O, R = ol.oracle(), ol.ref()
@@ -225,6 +232,7 @@ def test_static_table_rans():
 
 
 
+@needs_ref
 def test_find_lz_rgb_pinned_against_reference():
     """lz.hpp:6 — oracle restatement vs the compiled reference: LZ bytes and nuke map, every seek distance
     encode_tile uses (6, 10, 11, 12, 14) and every break-even bonus, on images that contain matches."""
@@ -245,6 +253,7 @@ def test_find_lz_rgb_pinned_against_reference():
 
 
 
+@needs_ref
 def test_lz_params_pinned_against_reference():
     rng = np.random.default_rng(5)
     for it in range(30):
@@ -259,6 +268,7 @@ def test_lz_params_pinned_against_reference():
         assert ol.oracle().orc_count_colours(img, img.size) == want == (ncol if ncol <= 256 else -1)
 
 
+@needs_ref
 def test_encode_tile_subgreen_with_lz_pinned_against_reference():
     """choh.cpp:104-382 at -s0 on photographic tiles with repeats: the oracle's pieces (find_lz_rgb, NUKE-aware
     layer_encode) assembled by encode_tile's rules give the reference's tile bytes."""
@@ -274,6 +284,7 @@ def test_encode_tile_subgreen_with_lz_pinned_against_reference():
     assert nuked > 50
 
 
+@needs_ref
 def test_encode_tile_all_modes_pinned_against_reference():
     """encode_tile at cruncher modes 1-4 (wider LZ windows, predictor search, prob_bits search, the plain-RGB
     alternative at modes 3-4) on photographic tiles with repeats; one tile is built so that plain RGB wins."""
