@@ -32,6 +32,8 @@ struct Buf {
     uint64_t epoch = 0;  // the top-level call (root context's `epoch`) that last asked for this buffer
 };
 
+constexpr int kPipeDepth = 4;  // most chunks in flight in a host-buffer call (hoh_*_images*_host)
+
 }  // namespace
 
 struct hoh_ctx {
@@ -51,13 +53,21 @@ struct hoh_ctx {
     size_t flush_bytes = 0;
     std::map<uint64_t, double*> e_tabs;  // plane size -> device table of -log2(f/size)
     bool smem_opt_in = false;
-    // host-buffer pipeline (hoh_*_images_s0_host): copy streams, events, pinned offset staging
+    // host-buffer pipeline of the four host calls (hoh_{en,de}code_images[_s0]_host): copy streams, per-slot events,
+    // pinned offset staging
     bool pipe_ready = false;
     cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-    cudaEvent_t ev_h2d[4] = {}, ev_comp[4] = {}, ev_d2h[4] = {}, ev_off[4] = {}, ev_start = nullptr;
-    uint64_t* h_off[4] = {nullptr, nullptr, nullptr, nullptr};
-    size_t h_off_cap[4] = {0, 0, 0, 0};
-    hoh_ctx* child[4] = {nullptr, nullptr, nullptr, nullptr};  // one per chunk in flight (own stream + scratch)
+    cudaEvent_t ev_h2d[kPipeDepth] = {}, ev_comp[kPipeDepth] = {}, ev_d2h[kPipeDepth] = {}, ev_off[kPipeDepth] = {};
+    cudaEvent_t ev_start = nullptr;
+    uint64_t* h_off[kPipeDepth] = {};
+    size_t h_off_cap[kPipeDepth] = {};
+    // Child contexts (own stream, own scratch), created on first use by child_of():
+    //   child[b]            slot b of the s0 host calls: codes its chunks and holds their staging
+    //   child[0], child[1]  the 8-bit / 9-bit layer_encode forks of hoh_encode_images
+    //   child[2], child[3]  staging of slots 0 / 1 of the whole-tile host calls
+    // new_shape() frees the scratch of ctx, child[0] and child[1], and the whole-tile host calls reach it from inside
+    // their pipeline, so whole-tile staging must never sit in one of those three.
+    hoh_ctx* child[4] = {};
     // Scratch of EARLIER top-level calls stays cached (the next call of the same kind reuses it) but is given back when an
     // allocation fails: the root context counts top-level calls (`epoch`, bumped by the outermost entry point: `depth`),
     // every buffer remembers the call that last asked for it, and scratch() frees the others before it gives up.
@@ -565,6 +575,16 @@ int new_shape(hoh_ctx* ctx, uint64_t key, bool decode) {
     slot = key;
     return HOH_OK;
 }
+
+// Child context k of ctx (roles: hoh_ctx::child), created on first use.
+int child_of(hoh_ctx* ctx, int k, hoh_ctx** out) {
+    if (!ctx->child[k]) {
+        if (hoh_ctx_create(ctx->device, nullptr, &ctx->child[k]) != HOH_OK) return HOH_E_CUDA;
+        ctx->child[k]->parent = ctx;
+    }
+    *out = ctx->child[k];
+    return HOH_OK;
+}
 }  // namespace
 
 // =================================================================================================
@@ -610,11 +630,11 @@ void hoh_ctx_destroy(hoh_ctx* ctx) {
             if (ev) cudaEventDestroy(ev);
     for (auto ev : ctx->prof_events) cudaEventDestroy(ev);
     for (auto ev : ctx->prof_pool) cudaEventDestroy(ev);
-    for (int k = 0; k < 4; k++)
-        if (ctx->child[k]) hoh_ctx_destroy(ctx->child[k]);
+    for (hoh_ctx* ch : ctx->child)
+        if (ch) hoh_ctx_destroy(ch);
     if (ctx->s_h2d) cudaStreamDestroy(ctx->s_h2d);
     if (ctx->s_d2h) cudaStreamDestroy(ctx->s_d2h);
-    for (int k = 0; k < 4; k++) {
+    for (int k = 0; k < kPipeDepth; k++) {
         if (ctx->ev_h2d[k]) cudaEventDestroy(ctx->ev_h2d[k]);
         if (ctx->ev_comp[k]) cudaEventDestroy(ctx->ev_comp[k]);
         if (ctx->ev_d2h[k]) cudaEventDestroy(ctx->ev_d2h[k]);
@@ -1056,27 +1076,45 @@ int hoh_decode_images_s0(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_by
     return HOH_OK;
 }
 
-// Host-buffer tile codec: the batch is cut into chunks that flow through a three-stage pipeline —
-// H2D copy (own stream), kernels, D2H copy (own stream) — so PCIe traffic in both directions overlaps
-// the kernels and each other.  The entropy kernels are bound by the serial chain of a stream, not by
-// how many streams run (one chunk alone takes almost as long as the whole batch), so the chunks'
-// kernels must themselves run CONCURRENTLY: each of the kPipeDepth chunks in flight has its own child
-// context (own stream, own scratch memory) and the GPU co-schedules their kernels.  The only host waits
-// are on the small per-chunk offset table (its total decides how many bytes to fetch).
-namespace {
-constexpr int kPipeDepth = 4;
+} // extern "C" (reopened below)
 
-// Whatever way a pipelined host call ends, nothing may still be reading or writing the caller's host buffers.
-struct PipeDrain {
+// Host-buffer tile codec: the batch is cut into chunks of whole images that flow through a three-stage pipeline —
+// H2D copy (own stream), kernels, D2H copy (own stream) — so PCIe traffic in both directions overlaps the kernels and
+// each other.  Chunk c goes through slot c % depth; a slot owns device staging, a pinned offset table and four events
+// that hand the staging from one stage to the next.  The host waits only on those small offset tables: an encoded
+// chunk's total decides how many bytes to fetch and where they go, and a decode slot's table is refilled on the host.
+// The s0 calls keep kPipeDepth chunks in flight.  Their entropy kernels are bound by the serial chain of a stream, not
+// by how many streams run (one chunk alone takes almost as long as the whole batch), so the chunks' kernels must
+// themselves run CONCURRENTLY: each slot codes on its own child context (own stream, own scratch memory) and the GPU
+// co-schedules their kernels.  The whole-tile calls keep two chunks in flight, coded on the context itself
+// (tile_chunk_plan gives the reason).
+namespace {
+
+// The context that codes a slot's chunks, the context whose scratch holds its device staging, that staging and the
+// pinned copy of its offset table.
+struct PipeSlot {
+    hoh_ctx* run = nullptr;
+    hoh_ctx* stage = nullptr;
+    uint8_t *rgb = nullptr, *packed = nullptr;
+    uint64_t *off = nullptr, *h_off = nullptr;
+    void* rec = nullptr;  // per-unit records: hoh_stream_result / hoh_tile_result (encode), int32_t status (decode)
+};
+
+// One host-buffer call: chunk c holds images bounds[c] .. bounds[c+1] and goes through slot c % depth.  A unit is one
+// entry of the offset table: a stream (s0 calls) or a tile (whole-tile calls).
+struct Pipe {
     hoh_ctx* ctx;
-    explicit PipeDrain(hoh_ctx* c) : ctx(c) {}
-    ~PipeDrain() {
-        if (ctx->s_h2d) cudaStreamSynchronize(ctx->s_h2d);
-        if (ctx->s_d2h) cudaStreamSynchronize(ctx->s_d2h);
-        cudaStreamSynchronize(ctx->stream);
-        for (hoh_ctx* ch : ctx->child)
-            if (ch) cudaStreamSynchronize(ch->stream);
+    std::vector<size_t> bounds;
+    size_t raw1, units, rec_bytes;  // per image: bytes of pixels and units; bytes of one unit's record
+    size_t max_chunk = 0;           // images in the largest chunk
+    int depth;
+    PipeSlot slot[kPipeDepth];
+    Pipe(hoh_ctx* c, std::vector<size_t> b, int max_depth, size_t raw_per_image, size_t units_per_image, size_t rec)
+        : ctx(c), bounds(std::move(b)), raw1(raw_per_image), units(units_per_image), rec_bytes(rec) {
+        for (size_t k = 0; k < chunks(); k++) max_chunk = std::max(max_chunk, bounds[k + 1] - bounds[k]);
+        depth = (int)std::min(chunks(), (size_t)max_depth);
     }
+    size_t chunks() const { return bounds.size() - 1; }
 };
 
 int pipe_init(hoh_ctx* ctx) {
@@ -1088,8 +1126,6 @@ int pipe_init(hoh_ctx* ctx) {
         CK(cudaEventCreateWithFlags(&ctx->ev_comp[k], cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&ctx->ev_d2h[k], cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&ctx->ev_off[k], cudaEventDisableTiming));
-        if (!ctx->child[k] && hoh_ctx_create(ctx->device, nullptr, &ctx->child[k]) != HOH_OK) return HOH_E_CUDA;
-        ctx->child[k]->parent = ctx;
     }
     CK(cudaEventCreateWithFlags(&ctx->ev_start, cudaEventDisableTiming));
     ctx->pipe_ready = true;
@@ -1118,19 +1154,18 @@ size_t chunk_images_for(size_t n_images, size_t raw_per_image) {
     if (per > n_images) per = n_images;
     return per;
 }
-// Chunk boundaries (image indices, n_chunks + 1 of them) of a pipelined host call.  What the pipeline cannot hide is its
+// Chunk boundaries (image indices, n_chunks + 1 of them) of an s0 host call.  What the pipeline cannot hide is its
 // head and its tail: before the first chunk's kernels have run nothing flows back, and the last chunk's kernels and
 // fetch run after the last byte has gone in.  A chunk's kernels last about as long whatever its size (one stream's
 // serial chain), so both ends are made of short chunks that double up to the steady size: per/8, per/4, per/2, per, ...,
 // per, per/2, per/4, per/8 (never below ~32 MB of pixels).
-std::vector<size_t> chunk_plan(size_t n_images, size_t raw_per_image, size_t* max_chunk) {
+std::vector<size_t> chunk_plan(size_t n_images, size_t raw_per_image) {
     const size_t per = chunk_images_for(n_images, raw_per_image);
     std::vector<size_t> bounds{0};
     const size_t floor_per = pipe_chunk_floor() / 2 / (raw_per_image ? raw_per_image : 1) + 1;
     std::vector<size_t> ramp;
-    if (!getenv("HOH_NO_RAMP"))
-        for (size_t r = std::max<size_t>(per / 8, 1); r < per; r *= 2)
-            if (r >= floor_per) ramp.push_back(r);
+    for (size_t r = std::max<size_t>(per / 8, 1); r < per; r *= 2)
+        if (r >= floor_per) ramp.push_back(r);
     size_t ramp_sum = 0;
     for (size_t r : ramp) ramp_sum += r;
     if (n_images < 2 * ramp_sum + 2 * per) {
@@ -1141,28 +1176,150 @@ std::vector<size_t> chunk_plan(size_t n_images, size_t raw_per_image, size_t* ma
     const size_t middle = n_images - 2 * ramp_sum, n_mid = (middle + per - 1) / per;
     for (size_t k = 0; k < n_mid; k++) bounds.push_back(bounds.back() + middle / n_mid + (k < middle % n_mid ? 1 : 0));
     for (size_t k = ramp.size(); k-- > 0;) bounds.push_back(bounds.back() + ramp[k]);
-    *max_chunk = 0;
-    for (size_t k = 0; k + 1 < bounds.size(); k++) *max_chunk = std::max(*max_chunk, bounds[k + 1] - bounds[k]);
     return bounds;
 }
-// everything queued on the parent's stream so far happens before the pipeline, and the pipeline's
-// completion is visible on the parent's stream afterwards
-int pipe_enter(hoh_ctx* ctx) {
+
+// Allocates every slot's staging (packed_cap bytes of payloads) and makes the copy streams and the slots' streams wait
+// for everything queued on the caller's stream so far.
+int pipe_begin(Pipe& pp, size_t packed_cap) {
+    hoh_ctx* ctx = pp.ctx;
+    TRY(pipe_init(ctx));
+    const size_t units = pp.max_chunk * pp.units;
+    for (int b = 0; b < pp.depth; b++) {
+        PipeSlot& s = pp.slot[b];
+        TRY(scratch_t(s.stage, S_IO_A, pp.max_chunk * pp.raw1, &s.rgb));
+        TRY(scratch_t(s.stage, S_IO_B, packed_cap, &s.packed));
+        TRY(scratch_t(s.stage, S_IO_C, units + 1, &s.off));
+        TRY(scratch(s.stage, S_IO_D, units * pp.rec_bytes, &s.rec));
+        TRY(pinned_off(ctx, b, units + 1, &s.h_off));
+    }
     CK(cudaEventRecord(ctx->ev_start, ctx->stream));
     CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_start, 0));
     CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_start, 0));
-    for (int k = 0; k < kPipeDepth; k++) CK(cudaStreamWaitEvent(ctx->child[k]->stream, ctx->ev_start, 0));
+    for (int b = 0; b < pp.depth; b++)
+        if (pp.slot[b].run != ctx) CK(cudaStreamWaitEvent(pp.slot[b].run->stream, ctx->ev_start, 0));
     return HOH_OK;
 }
-int pipe_leave(hoh_ctx* ctx, uint64_t* launches_before) {
-    CK(cudaStreamSynchronize(ctx->s_d2h));
-    for (int k = 0; k < kPipeDepth; k++) {
-        CK(cudaStreamSynchronize(ctx->child[k]->stream));
-        ctx->launches += ctx->child[k]->launches - launches_before[k];
+
+// Whatever way a host-buffer call ends, nothing may still read or write the caller's buffers when it returns.  The
+// slots' child contexts launch on the caller's behalf: their launches count as the caller's.
+struct PipeGuard {
+    const Pipe& pp;
+    uint64_t launches[kPipeDepth];
+    explicit PipeGuard(const Pipe& p) : pp(p) {
+        for (int b = 0; b < pp.depth; b++) launches[b] = pp.slot[b].run->launches;
     }
+    ~PipeGuard() {
+        hoh_ctx* ctx = pp.ctx;
+        cudaStreamSynchronize(ctx->s_h2d);
+        cudaStreamSynchronize(ctx->s_d2h);
+        cudaStreamSynchronize(ctx->stream);
+        for (hoh_ctx* ch : ctx->child)
+            if (ch) cudaStreamSynchronize(ch->stream);
+        for (int b = 0; b < pp.depth; b++)
+            if (pp.slot[b].run != ctx) ctx->launches += pp.slot[b].run->launches - launches[b];
+    }
+};
+
+// Encodes the chunks of a host-buffer call.  code(b, n_images) codes the chunk in slot b on the slot's run context:
+// pixels in rgb, payloads to packed (dev_cap bytes), chunk-relative offsets to off, records to rec.  Chunk c's H2D copy
+// and kernels are queued depth - 1 chunks ahead of the fetch of its payloads.  off_host receives the offsets into
+// packed_host, rec_host (may be NULL) the records, chunk_base (may be NULL) where each chunk starts in packed_host.
+template <class Code>
+int pipe_encode(Pipe& pp, size_t dev_cap, const uint8_t* rgb_host, uint8_t* packed_host, size_t packed_cap,
+                uint64_t* off_host, void* rec_host, uint64_t* chunk_base, Code code) {
+    hoh_ctx* ctx = pp.ctx;
+    TRY(pipe_begin(pp, dev_cap));
+    PipeGuard guard(pp);
+    const size_t n_chunks = pp.chunks(), depth = pp.depth, units = pp.units;
+    uint64_t base = 0;
+    off_host[0] = 0;
+    for (size_t c = 0; c + 1 < n_chunks + depth; c++) {
+        if (c < n_chunks) {  // copy in and code chunk c
+            const int b = (int)(c % depth);
+            const PipeSlot& s = pp.slot[b];
+            const size_t first = pp.bounds[c], n_c = pp.bounds[c + 1] - first;
+            if (c >= depth) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // s.rgb consumed
+            CK(cudaMemcpyAsync(s.rgb, rgb_host + first * pp.raw1, n_c * pp.raw1, cudaMemcpyHostToDevice, ctx->s_h2d));
+            CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
+            CK(cudaStreamWaitEvent(s.run->stream, ctx->ev_h2d[b], 0));
+            if (c >= depth) CK(cudaStreamWaitEvent(s.run->stream, ctx->ev_d2h[b], 0));  // s.packed fetched
+            TRY(code(b, n_c));
+            CK(cudaEventRecord(ctx->ev_comp[b], s.run->stream));
+            // its offset table follows on the run stream (tiny; must not queue behind big fetches)
+            CK(cudaMemcpyAsync(s.h_off, s.off, (n_c * units + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.run->stream));
+            CK(cudaEventRecord(ctx->ev_off[b], s.run->stream));
+        }
+        if (c + 1 >= depth) {  // fetch chunk p = c - (depth - 1)
+            const size_t p = c + 1 - depth;
+            const int b = (int)(p % depth);
+            const PipeSlot& s = pp.slot[b];
+            const size_t u0 = pp.bounds[p] * units, nu = pp.bounds[p + 1] * units - u0;
+            CK(cudaEventSynchronize(ctx->ev_off[b]));
+            const uint64_t total = s.h_off[nu];
+            if (total > dev_cap || base + total > packed_cap) return HOH_E_CAPACITY;
+            CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[b], 0));
+            CK(cudaMemcpyAsync(packed_host + base, s.packed, total, cudaMemcpyDeviceToHost, ctx->s_d2h));
+            if (rec_host)
+                CK(cudaMemcpyAsync(static_cast<uint8_t*>(rec_host) + u0 * pp.rec_bytes, s.rec, nu * pp.rec_bytes,
+                                   cudaMemcpyDeviceToHost, ctx->s_d2h));
+            CK(cudaEventRecord(ctx->ev_d2h[b], ctx->s_d2h));
+            for (size_t i = 1; i <= nu; i++) off_host[u0 + i] = base + s.h_off[i];
+            if (chunk_base) chunk_base[p] = base;
+            base += total;
+        }
+    }
+    CK(cudaStreamSynchronize(ctx->s_d2h));
+    return HOH_OK;
+}
+
+// Decodes the chunks of a host-buffer call.  code(b, n_images, packed_bytes) decodes the chunk in slot b on the slot's
+// run context: payloads in packed (packed_bytes, zero padding included), chunk-relative offsets in off, pixels to rgb,
+// per-unit status to rec.  Per chunk: rebase its offsets on the host, pad, H2D payloads and offsets, code, D2H pixels
+// and status.  Offsets that decrease from one chunk to the next or end beyond packed_bytes are HOH_E_ARG.
+template <class Code>
+int pipe_decode(Pipe& pp, const uint8_t* packed_host, size_t packed_bytes, const uint64_t* off_host, uint8_t* rgb_host,
+                int32_t* status_host, Code code) {
+    hoh_ctx* ctx = pp.ctx;
+    const size_t n_chunks = pp.chunks(), depth = pp.depth, units = pp.units;
+    size_t max_packed = 0;
+    for (size_t c = 0; c < n_chunks; c++) {
+        const uint64_t lo = off_host[pp.bounds[c] * units], hi = off_host[pp.bounds[c + 1] * units];
+        if (hi < lo || hi > packed_bytes) return HOH_E_ARG;
+        max_packed = std::max<size_t>(max_packed, hi - lo);
+    }
+    // >= 32 zero bytes behind a chunk's last payload byte (the decode input contract, hohgpu.h)
+    auto padded = [](size_t bytes) { return (bytes + 47) & ~(size_t)15; };
+    TRY(pipe_begin(pp, padded(max_packed)));
+    PipeGuard guard(pp);
+    for (size_t c = 0; c < n_chunks; c++) {
+        const int b = (int)(c % depth);
+        const PipeSlot& s = pp.slot[b];
+        const size_t first = pp.bounds[c], n_c = pp.bounds[c + 1] - first, u0 = first * units, nu = n_c * units;
+        const uint64_t lo = off_host[u0], bytes = off_host[u0 + nu] - lo;
+        const size_t aligned = bytes & ~(size_t)15;
+        if (c >= depth) CK(cudaEventSynchronize(ctx->ev_h2d[b]));  // s.h_off was read by chunk c-depth's copy
+        for (size_t i = 0; i <= nu; i++) s.h_off[i] = off_host[u0 + i] - lo;
+        if (c >= depth) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // s.packed / s.off consumed
+        CK(cudaMemsetAsync(s.packed + aligned, 0, padded(bytes) - aligned, ctx->s_h2d));
+        CK(cudaMemcpyAsync(s.packed, packed_host + lo, bytes, cudaMemcpyHostToDevice, ctx->s_h2d));
+        CK(cudaMemcpyAsync(s.off, s.h_off, (nu + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->s_h2d));
+        CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
+        CK(cudaStreamWaitEvent(s.run->stream, ctx->ev_h2d[b], 0));
+        if (c >= depth) CK(cudaStreamWaitEvent(s.run->stream, ctx->ev_d2h[b], 0));  // s.rgb fetched
+        TRY(code(b, n_c, padded(bytes)));
+        CK(cudaEventRecord(ctx->ev_comp[b], s.run->stream));
+        CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[b], 0));
+        CK(cudaMemcpyAsync(rgb_host + first * pp.raw1, s.rgb, n_c * pp.raw1, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        if (status_host)
+            CK(cudaMemcpyAsync(status_host + u0, s.rec, nu * pp.rec_bytes, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        CK(cudaEventRecord(ctx->ev_d2h[b], ctx->s_d2h));
+    }
+    CK(cudaStreamSynchronize(ctx->s_d2h));
     return HOH_OK;
 }
 }  // namespace
+extern "C" {
 
 int hoh_encode_images_s0_host(hoh_ctx* ctx, const uint8_t* rgb_host, size_t n_images, uint32_t width,
                               uint32_t height, uint8_t* packed_host, size_t packed_cap, uint64_t* off_host,
@@ -1172,75 +1329,22 @@ int hoh_encode_images_s0_host(hoh_ctx* ctx, const uint8_t* rgb_host, size_t n_im
     if (n_images == 0) return HOH_OK;
     hoh_tile_geometry hg;
     TRY(hoh_tile_geometry_for(width, height, &hg));
-    TRY(pipe_init(ctx));
     const size_t raw1 = (size_t)width * height * 3;
-    size_t per;  // the largest chunk
-    const std::vector<size_t> bounds = chunk_plan(n_images, raw1, &per);
-    const size_t n_chunks = bounds.size() - 1;
-    const size_t spi = hg.streams_per_image;
-    const size_t chunk_streams = per * spi;
-    const size_t out_bytes = hoh_encode_images_out_bytes(&hg, per);
-    const size_t dev_packed_cap = per * raw1 + per * raw1 / 4 + 4096 * chunk_streams;
-    const int depth = (int)(n_chunks < (size_t)kPipeDepth ? n_chunks : kPipeDepth);
-    uint8_t *d_rgb[kPipeDepth], *d_packed[kPipeDepth], *d_out[kPipeDepth];
-    hoh_stream_result* d_res[kPipeDepth];
-    uint64_t *d_off[kPipeDepth], *h_off[kPipeDepth];
-    uint64_t launches_before[kPipeDepth];
-    for (int k = 0; k < kPipeDepth; k++) launches_before[k] = ctx->child[k]->launches;
-    for (int k = 0; k < depth; k++) {  // staging lives in the child contexts
-        hoh_ctx* ch = ctx->child[k];
-        TRY(scratch_t(ch, S_IO_A, per * raw1, &d_rgb[k]));
-        TRY(scratch_t(ch, S_IO_B, out_bytes, &d_out[k]));
-        TRY(scratch_t(ch, S_IO_C, dev_packed_cap, &d_packed[k]));
-        TRY(scratch_t(ch, S_IO_D, chunk_streams + 1, &d_off[k]));
-        TRY(scratch_t(ch, S_RESULTS, chunk_streams, &d_res[k]));
-        TRY(pinned_off(ctx, k, chunk_streams + 1, &h_off[k]));
+    Pipe pp(ctx, chunk_plan(n_images, raw1), kPipeDepth, raw1, hg.streams_per_image, sizeof(hoh_stream_result));
+    const size_t per = pp.max_chunk, out_bytes = hoh_encode_images_out_bytes(&hg, per);
+    const size_t dev_cap = per * raw1 + per * raw1 / 4 + 4096 * per * pp.units;
+    uint8_t* d_out[kPipeDepth];  // the slabs hoh_encode_images_s0 codes into before it gathers the payloads
+    for (int b = 0; b < pp.depth; b++) {  // slot b codes on child[b], from staging there
+        TRY(child_of(ctx, b, &pp.slot[b].run));
+        pp.slot[b].stage = pp.slot[b].run;
+        TRY(scratch_t(pp.slot[b].stage, S_IO_E, out_bytes, &d_out[b]));
     }
-    TRY(pipe_enter(ctx));
-    PipeDrain drain(ctx);
-    uint64_t base = 0;
-    off_host[0] = 0;
-    // chunk c: (1) H2D + kernels are queued `depth - 1` chunks ahead of (2) the fetch of its payloads
-    for (size_t c = 0; c < n_chunks + (size_t)depth - 1 + 1; c++) {
-        if (c < n_chunks) {
-            const int b = (int)(c % depth);
-            hoh_ctx* ch = ctx->child[b];
-            const size_t first = bounds[c], n_c = bounds[c + 1] - first;
-            if (c >= (size_t)depth) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // d_rgb[b] free again
-            CK(cudaMemcpyAsync(d_rgb[b], rgb_host + first * raw1, n_c * raw1, cudaMemcpyHostToDevice, ctx->s_h2d));
-            CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
-            CK(cudaStreamWaitEvent(ch->stream, ctx->ev_h2d[b], 0));
-            if (c >= (size_t)depth) CK(cudaStreamWaitEvent(ch->stream, ctx->ev_d2h[b], 0));  // d_packed[b] fetched
-            TRY(hoh_encode_images_s0(ch, d_rgb[b], n_c, width, height, nullptr, d_out[b], out_bytes, d_res[b], d_packed[b],
-                                     dev_packed_cap, d_off[b]));
-            CK(cudaEventRecord(ctx->ev_comp[b], ch->stream));
-            // its offset table follows on the child's own stream (tiny; must not queue behind big fetches)
-            CK(cudaMemcpyAsync(h_off[b], d_off[b], (n_c * spi + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ch->stream));
-            CK(cudaEventRecord(ctx->ev_off[b], ch->stream));
-        }
-        if (c + 1 >= (size_t)depth && c + 1 - depth < n_chunks) {  // fetch chunk p = c - (depth - 1)
-            const size_t pc = c + 1 - depth;
-            const int p = (int)(pc % depth);
-            const size_t pfirst = bounds[pc], n_p = bounds[pc + 1] - pfirst;
-            CK(cudaEventSynchronize(ctx->ev_off[p]));
-            const uint64_t total = h_off[p][n_p * spi];
-            if (base + total > packed_cap || total > dev_packed_cap) {
-                uint64_t dummy[kPipeDepth];
-                for (int k = 0; k < kPipeDepth; k++) dummy[k] = ctx->child[k]->launches;
-                pipe_leave(ctx, dummy);
-                return HOH_E_CAPACITY;
-            }
-            CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[p], 0));
-            CK(cudaMemcpyAsync(packed_host + base, d_packed[p], total, cudaMemcpyDeviceToHost, ctx->s_d2h));
-            if (results_host)
-                CK(cudaMemcpyAsync(results_host + pfirst * spi, d_res[p], n_p * spi * sizeof(hoh_stream_result),
-                                   cudaMemcpyDeviceToHost, ctx->s_d2h));
-            CK(cudaEventRecord(ctx->ev_d2h[p], ctx->s_d2h));
-            for (size_t i = 1; i <= n_p * spi; i++) off_host[pfirst * spi + i] = base + h_off[p][i];
-            base += total;
-        }
-    }
-    return pipe_leave(ctx, launches_before);
+    return pipe_encode(pp, dev_cap, rgb_host, packed_host, packed_cap, off_host, results_host, nullptr,
+                       [&](int b, size_t n_c) {
+                           const PipeSlot& s = pp.slot[b];
+                           return hoh_encode_images_s0(s.run, s.rgb, n_c, width, height, nullptr, d_out[b], out_bytes,
+                                                       static_cast<hoh_stream_result*>(s.rec), s.packed, dev_cap, s.off);
+                       });
 }
 
 int hoh_decode_images_s0_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t packed_bytes,
@@ -1251,61 +1355,18 @@ int hoh_decode_images_s0_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t p
     if (n_images == 0) return HOH_OK;
     hoh_tile_geometry hg;
     TRY(hoh_tile_geometry_for(width, height, &hg));
-    TRY(pipe_init(ctx));
     const size_t raw1 = (size_t)width * height * 3;
-    size_t per;  // the largest chunk
-    const std::vector<size_t> bounds = chunk_plan(n_images, raw1, &per);
-    const size_t n_chunks = bounds.size() - 1;
-    const size_t spi = hg.streams_per_image;
-    const size_t chunk_streams = per * spi;
-    size_t max_packed = 0;  // largest packed chunk
-    for (size_t c = 0; c < n_chunks; c++) {
-        const size_t s0 = bounds[c] * spi, s1 = bounds[c + 1] * spi;
-        if (off_host[s1] < off_host[s0] || off_host[s1] > packed_bytes) return HOH_E_ARG;
-        if (off_host[s1] - off_host[s0] > max_packed) max_packed = off_host[s1] - off_host[s0];
+    Pipe pp(ctx, chunk_plan(n_images, raw1), kPipeDepth, raw1, hg.streams_per_image, sizeof(int32_t));
+    for (int b = 0; b < pp.depth; b++) {  // slot b decodes on child[b], from staging there
+        TRY(child_of(ctx, b, &pp.slot[b].run));
+        pp.slot[b].stage = pp.slot[b].run;
     }
-    const size_t padded_cap = (max_packed + 47) & ~(size_t)15;
-    const int depth = (int)(n_chunks < (size_t)kPipeDepth ? n_chunks : kPipeDepth);
-    uint8_t *d_rgb[kPipeDepth], *d_packed[kPipeDepth];
-    uint64_t *d_off[kPipeDepth], *h_off[kPipeDepth];
-    int32_t* d_st[kPipeDepth];
-    uint64_t launches_before[kPipeDepth];
-    for (int k = 0; k < kPipeDepth; k++) launches_before[k] = ctx->child[k]->launches;
-    for (int k = 0; k < depth; k++) {
-        hoh_ctx* ch = ctx->child[k];
-        TRY(scratch_t(ch, S_IO_A, per * raw1, &d_rgb[k]));
-        TRY(scratch_t(ch, S_IO_C, padded_cap, &d_packed[k]));
-        TRY(scratch_t(ch, S_IO_D, chunk_streams + 1, &d_off[k]));
-        TRY(scratch_t(ch, S_IO_E, chunk_streams, &d_st[k]));
-        TRY(pinned_off(ctx, k, chunk_streams + 1, &h_off[k]));
-    }
-    TRY(pipe_enter(ctx));
-    PipeDrain drain(ctx);
-    for (size_t c = 0; c < n_chunks; c++) {
-        const int b = (int)(c % depth);
-        hoh_ctx* ch = ctx->child[b];
-        const size_t first = bounds[c], n_c = bounds[c + 1] - first;
-        const size_t s0 = first * spi, ns = n_c * spi;
-        const uint64_t lo = off_host[s0], bytes = off_host[s0 + ns] - lo;
-        const size_t padded = (bytes + 47) & ~(size_t)15;
-        if (c >= (size_t)depth) CK(cudaEventSynchronize(ctx->ev_h2d[b]));  // h_off[b] was read by chunk c-depth's copy
-        for (size_t i = 0; i <= ns; i++) h_off[b][i] = off_host[s0 + i] - lo;
-        if (c >= (size_t)depth) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // d_packed[b] / d_off[b] free
-        CK(cudaMemsetAsync(d_packed[b] + (bytes & ~(size_t)15), 0, padded - (bytes & ~(size_t)15), ctx->s_h2d));
-        CK(cudaMemcpyAsync(d_packed[b], packed_host + lo, bytes, cudaMemcpyHostToDevice, ctx->s_h2d));
-        CK(cudaMemcpyAsync(d_off[b], h_off[b], (ns + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->s_h2d));
-        CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
-        CK(cudaStreamWaitEvent(ch->stream, ctx->ev_h2d[b], 0));
-        if (c >= (size_t)depth) CK(cudaStreamWaitEvent(ch->stream, ctx->ev_d2h[b], 0));  // d_rgb[b] fetched
-        TRY(hoh_decode_images_s0(ch, d_packed[b], padded, d_off[b], n_c, width, height, nullptr, d_rgb[b], d_st[b]));
-        CK(cudaEventRecord(ctx->ev_comp[b], ch->stream));
-        CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[b], 0));
-        CK(cudaMemcpyAsync(rgb_host + first * raw1, d_rgb[b], n_c * raw1, cudaMemcpyDeviceToHost, ctx->s_d2h));
-        if (status_host)
-            CK(cudaMemcpyAsync(status_host + s0, d_st[b], ns * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->s_d2h));
-        CK(cudaEventRecord(ctx->ev_d2h[b], ctx->s_d2h));
-    }
-    return pipe_leave(ctx, launches_before);
+    return pipe_decode(pp, packed_host, packed_bytes, off_host, rgb_host, status_host,
+                       [&](int b, size_t n_c, size_t padded) {
+                           const PipeSlot& s = pp.slot[b];
+                           return hoh_decode_images_s0(s.run, s.packed, padded, s.off, n_c, width, height, nullptr,
+                                                       s.rgb, static_cast<int32_t*>(s.rec));
+                       });
 }
 
 // =================================================================================================
@@ -1911,12 +1972,8 @@ int hoh_encode_images(hoh_ctx* ctx, const uint8_t* d_rgb, size_t n_images, uint3
             hoh_ctx* c8 = ctx;
             hoh_ctx* c9 = ctx;
             if (!ctx->profiling) {
-                for (int k = 0; k < 2; k++) {
-                    if (!ctx->child[k] && hoh_ctx_create(ctx->device, nullptr, &ctx->child[k]) != HOH_OK) return HOH_E_CUDA;
-                    ctx->child[k]->parent = ctx;
-                }
-                c8 = ctx->child[0];
-                c9 = ctx->child[1];
+                TRY(child_of(ctx, 0, &c8));
+                TRY(child_of(ctx, 1, &c9));
                 TRY(aux_init(ctx));
                 CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
                 CK(cudaStreamWaitEvent(c8->stream, ctx->ev_fork, 0));
@@ -2053,13 +2110,13 @@ int hoh_decode_images(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_bytes
 // -------------------------------------------------------------------------------------------------
 } // extern "C" (reopened below)
 namespace {
-// Images per chunk of a whole-tile host call.  The mode >= 1 kernels (rANS candidates, the plane walks of the decoder) last
-// as long as ONE stream's serial chain however few streams a launch holds, so cutting a batch into k chunks multiplies
-// their time by almost k (BASELINE config 3, decode: 112 ms for 256 frames at once, 4 x ~100 ms in four chunks) while
-// the copies it would hide are short (6.4 GB at 55 GB/s = 116 ms).  Two chunks: the second one's H2D and the first
-// one's D2H overlap the kernels, and the chain is paid twice, not four times; one chunk when the batch is small.  The
-// double-buffered staging (raw + packed, twice) must leave most of the device to the codec's own scratch.
-size_t tile_chunk_images(size_t n_images, size_t raw_per_image) {
+// Chunk boundaries (image indices) of a whole-tile host call.  The mode >= 1 kernels (rANS candidates, the plane walks of
+// the decoder) last as long as ONE stream's serial chain however few streams a launch holds, so cutting a batch into k
+// chunks multiplies their time by almost k (BASELINE config 3, decode: 112 ms for 256 frames at once, 4 x ~100 ms in four
+// chunks) while the copies it would hide are short (6.4 GB at 55 GB/s = 116 ms).  Two chunks: the second one's H2D and
+// the first one's D2H overlap the kernels, and the chain is paid twice, not four times; one chunk when the batch is
+// small.  The double-buffered staging (raw + packed, twice) must leave most of the device to the codec's own scratch.
+std::vector<size_t> tile_chunk_plan(size_t n_images, size_t raw_per_image) {
     size_t per = (n_images + 1) / 2;
     const size_t min_per = (256u << 20) / (raw_per_image ? raw_per_image : 1) + 1;
     if (per < min_per) per = min_per;
@@ -2069,7 +2126,10 @@ size_t tile_chunk_images(size_t n_images, size_t raw_per_image) {
         if (cap >= 1 && per > cap) per = cap;
     }
     if (per > n_images) per = n_images;
-    return per ? per : 1;
+    if (per == 0) per = 1;
+    std::vector<size_t> bounds{0};
+    while (bounds.back() < n_images) bounds.push_back(std::min(bounds.back() + per, n_images));
+    return bounds;
 }
 }  // namespace
 extern "C" {
@@ -2083,76 +2143,22 @@ int hoh_encode_images_host(hoh_ctx* ctx, const uint8_t* rgb_host, size_t n_image
     if (n_images == 0) return HOH_OK;
     hoh_tile_geometry hg;
     TRY(hoh_tile_geometry_for(width, height, &hg));
-    TRY(pipe_init(ctx));
-    const size_t raw1 = (size_t)width * height * 3, tpi = hg.tiles_per_image;
-    const size_t per = tile_chunk_images(n_images, raw1);
-    const size_t n_chunks = (n_images + per - 1) / per;
-    const size_t chunk_tiles = per * tpi;
-    const size_t dev_cap = per * raw1 + per * raw1 / 2 + 8192 * chunk_tiles;
-    constexpr int kBuf = 2;
-    uint8_t *d_rgb[kBuf], *d_packed[kBuf];
-    uint64_t *d_off[kBuf], *h_off[kBuf];
-    hoh_tile_result* d_tiles[kBuf];
-    const int nbuf = n_chunks < (size_t)kBuf ? (int)n_chunks : kBuf;
-    hoh_ctx* stage = ctx->child[2];  // staging lives in a child that the codec itself never uses (it forks into child 0/1)
-    {
-        uint8_t *rgb2, *packed2;
-        uint64_t* off2;
-        hoh_tile_result* tiles2;
-        TRY(scratch_t(stage, S_IO_A, nbuf * per * raw1, &rgb2));
-        TRY(scratch_t(stage, S_IO_B, nbuf * dev_cap, &packed2));
-        TRY(scratch_t(stage, S_IO_C, nbuf * (chunk_tiles + 1), &off2));
-        TRY(scratch_t(stage, S_IO_D, nbuf * chunk_tiles, &tiles2));
-        for (int k = 0; k < nbuf; k++) {
-            d_rgb[k] = rgb2 + (size_t)k * per * raw1;
-            d_packed[k] = packed2 + (size_t)k * dev_cap;
-            d_off[k] = off2 + (size_t)k * (chunk_tiles + 1);
-            d_tiles[k] = tiles2 + (size_t)k * chunk_tiles;
-            TRY(pinned_off(ctx, k, chunk_tiles + 1, &h_off[k]));
-        }
+    const size_t raw1 = (size_t)width * height * 3;
+    Pipe pp(ctx, tile_chunk_plan(n_images, raw1), 2, raw1, hg.tiles_per_image, sizeof(hoh_tile_result));
+    for (int b = 0; b < pp.depth; b++) {  // coded on ctx itself, staging out of new_shape's reach (hoh_ctx::child)
+        pp.slot[b].run = ctx;
+        TRY(child_of(ctx, 2 + b, &pp.slot[b].stage));
     }
-    PipeDrain drain(ctx);
-    CK(cudaEventRecord(ctx->ev_start, ctx->stream));
-    CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_start, 0));
-    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_start, 0));
-    std::vector<uint64_t> chunk_base(n_chunks, 0);
-    uint64_t base = 0;
-    for (size_t c = 0; c <= n_chunks; c++) {
-        if (c < n_chunks) {  // copy in and code chunk c
-            const int b = (int)(c % nbuf);
-            const size_t first = c * per, n_c = std::min(per, n_images - first);
-            if (c >= (size_t)nbuf) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // d_rgb[b] consumed
-            CK(cudaMemcpyAsync(d_rgb[b], rgb_host + first * raw1, n_c * raw1, cudaMemcpyHostToDevice, ctx->s_h2d));
-            CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
-            CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_h2d[b], 0));
-            if (c >= (size_t)nbuf) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[b], 0));  // d_packed[b] fetched
-            TRY(hoh_encode_images(ctx, d_rgb[b], n_c, width, height, mode, flags, d_packed[b], dev_cap, d_off[b], d_tiles[b]));
-            CK(cudaEventRecord(ctx->ev_comp[b], ctx->stream));
-            CK(cudaMemcpyAsync(h_off[b], d_off[b], (n_c * tpi + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaEventRecord(ctx->ev_off[b], ctx->stream));
-        }
-        if (c >= 1) {  // fetch chunk c-1 while chunk c is being coded
-            const size_t pc = c - 1;
-            const int p = (int)(pc % nbuf);
-            const size_t pfirst = pc * per, n_p = std::min(per, n_images - pfirst);
-            CK(cudaEventSynchronize(ctx->ev_off[p]));
-            const uint64_t total = h_off[p][n_p * tpi];
-            if (total > dev_cap || base + total > packed_cap) return HOH_E_CAPACITY;
-            CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[p], 0));
-            CK(cudaMemcpyAsync(packed_host + base, d_packed[p], total, cudaMemcpyDeviceToHost, ctx->s_d2h));
-            CK(cudaMemcpyAsync(tiles_host + pfirst * tpi, d_tiles[p], n_p * tpi * sizeof(hoh_tile_result),
-                               cudaMemcpyDeviceToHost, ctx->s_d2h));
-            CK(cudaEventRecord(ctx->ev_d2h[p], ctx->s_d2h));
-            for (size_t i = 1; i <= n_p * tpi; i++) tile_off_host[pfirst * tpi + i] = base + h_off[p][i];
-            chunk_base[pc] = base;
-            base += total;
-        }
-    }
-    CK(cudaStreamSynchronize(ctx->s_d2h));
-    for (size_t c = 0; c < n_chunks; c++) {  // tile records carry chunk-relative offsets: rebase
-        const size_t first = c * per * tpi, cnt = std::min(per, n_images - c * per) * tpi;
-        for (size_t i = 0; i < cnt; i++) tiles_host[first + i].start += chunk_base[c];
-    }
+    const size_t per = pp.max_chunk, dev_cap = per * raw1 + per * raw1 / 2 + 8192 * per * pp.units;
+    std::vector<uint64_t> chunk_base(pp.chunks());
+    TRY(pipe_encode(pp, dev_cap, rgb_host, packed_host, packed_cap, tile_off_host, tiles_host, chunk_base.data(),
+                    [&](int b, size_t n_c) {
+                        const PipeSlot& s = pp.slot[b];
+                        return hoh_encode_images(ctx, s.rgb, n_c, width, height, mode, flags, s.packed, dev_cap, s.off,
+                                                 static_cast<hoh_tile_result*>(s.rec));
+                    }));
+    for (size_t c = 0; c < pp.chunks(); c++)  // tile records carry chunk-relative offsets: rebase
+        for (size_t t = pp.bounds[c] * pp.units; t < pp.bounds[c + 1] * pp.units; t++) tiles_host[t].start += chunk_base[c];
     return HOH_OK;
 }
 
@@ -2163,70 +2169,20 @@ int hoh_decode_images_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t pack
     if (n_images == 0) return HOH_OK;
     hoh_tile_geometry hg;
     TRY(hoh_tile_geometry_for(width, height, &hg));
-    TRY(pipe_init(ctx));
-    const size_t raw1 = (size_t)width * height * 3, tpi = hg.tiles_per_image;
-    const size_t per = tile_chunk_images(n_images, raw1);
-    const size_t n_chunks = (n_images + per - 1) / per;
-    const size_t chunk_tiles = per * tpi;
-    size_t max_packed = 0;
-    for (size_t c = 0; c < n_chunks; c++) {
-        const size_t t0 = c * chunk_tiles, t1 = std::min((c + 1) * per, n_images) * tpi;
-        if (tile_off_host[t1] < tile_off_host[t0] || tile_off_host[t1] > packed_bytes) return HOH_E_ARG;
-        max_packed = std::max<size_t>(max_packed, tile_off_host[t1] - tile_off_host[t0]);
+    const size_t raw1 = (size_t)width * height * 3;
+    Pipe pp(ctx, tile_chunk_plan(n_images, raw1), 2, raw1, hg.tiles_per_image, sizeof(int32_t));
+    for (int b = 0; b < pp.depth; b++) {  // decoded on ctx itself, staging out of new_shape's reach (hoh_ctx::child)
+        pp.slot[b].run = ctx;
+        TRY(child_of(ctx, 2 + b, &pp.slot[b].stage));
     }
-    const size_t padded_cap = (max_packed + 63) & ~(size_t)15;
-    constexpr int kBuf = 2;
-    const int nbuf = n_chunks < (size_t)kBuf ? (int)n_chunks : kBuf;
-    hoh_ctx* stage = ctx->child[2];
-    uint8_t *d_rgb[kBuf], *d_packed[kBuf];
-    uint64_t *d_off[kBuf], *h_off[kBuf];
-    int32_t* d_st[kBuf];
-    {
-        uint8_t *rgb2, *packed2;
-        uint64_t* off2;
-        int32_t* st2;
-        TRY(scratch_t(stage, S_IO_A, nbuf * per * raw1, &rgb2));
-        TRY(scratch_t(stage, S_IO_B, nbuf * padded_cap, &packed2));
-        TRY(scratch_t(stage, S_IO_C, nbuf * (chunk_tiles + 1), &off2));
-        TRY(scratch_t(stage, S_IO_D, nbuf * chunk_tiles, &st2));
-        for (int k = 0; k < nbuf; k++) {
-            d_rgb[k] = rgb2 + (size_t)k * per * raw1;
-            d_packed[k] = packed2 + (size_t)k * padded_cap;
-            d_off[k] = off2 + (size_t)k * (chunk_tiles + 1);
-            d_st[k] = st2 + (size_t)k * chunk_tiles;
-            TRY(pinned_off(ctx, k, chunk_tiles + 1, &h_off[k]));
-        }
-    }
-    PipeDrain drain(ctx);
-    CK(cudaEventRecord(ctx->ev_start, ctx->stream));
-    CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_start, 0));
-    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_start, 0));
-    for (size_t c = 0; c < n_chunks; c++) {
-        const int b = (int)(c % nbuf);
-        const size_t first = c * per, n_c = std::min(per, n_images - first);
-        const size_t t0 = first * tpi, nt = n_c * tpi;
-        const uint64_t lo = tile_off_host[t0], bytes = tile_off_host[t0 + nt] - lo;
-        const size_t padded = (bytes + 47) & ~(size_t)15;  // >= 32 zero bytes behind the last tile (hohgpu.h, decode contract)
-        if (c >= (size_t)nbuf) CK(cudaEventSynchronize(ctx->ev_h2d[b]));  // h_off[b] was read by chunk c-nbuf's copy
-        for (size_t i = 0; i <= nt; i++) h_off[b][i] = tile_off_host[t0 + i] - lo;
-        if (c >= (size_t)nbuf) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // d_packed[b] / d_off[b] consumed
-        CK(cudaMemsetAsync(d_packed[b] + (bytes & ~(size_t)15), 0, padded - (bytes & ~(size_t)15), ctx->s_h2d));
-        CK(cudaMemcpyAsync(d_packed[b], packed_host + lo, bytes, cudaMemcpyHostToDevice, ctx->s_h2d));
-        CK(cudaMemcpyAsync(d_off[b], h_off[b], (nt + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->s_h2d));
-        CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
-        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_h2d[b], 0));
-        if (c >= (size_t)nbuf) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[b], 0));  // d_rgb[b] fetched
-        // a tile that fails to decode leaves its pixels untouched: make "untouched" mean zero
-        CK(cudaMemsetAsync(d_rgb[b], 0, n_c * raw1, ctx->stream));
-        TRY(hoh_decode_images(ctx, d_packed[b], padded, d_off[b], n_c, width, height, d_rgb[b], d_st[b]));
-        CK(cudaEventRecord(ctx->ev_comp[b], ctx->stream));
-        CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[b], 0));
-        CK(cudaMemcpyAsync(rgb_host + first * raw1, d_rgb[b], n_c * raw1, cudaMemcpyDeviceToHost, ctx->s_d2h));
-        CK(cudaMemcpyAsync(status_host + t0, d_st[b], nt * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->s_d2h));
-        CK(cudaEventRecord(ctx->ev_d2h[b], ctx->s_d2h));
-    }
-    CK(cudaStreamSynchronize(ctx->s_d2h));
-    return HOH_OK;
+    return pipe_decode(pp, packed_host, packed_bytes, tile_off_host, rgb_host, status_host,
+                       [&](int b, size_t n_c, size_t padded) {
+                           const PipeSlot& s = pp.slot[b];
+                           // a tile that fails to decode leaves its pixels untouched: make "untouched" mean zero
+                           CK(cudaMemsetAsync(s.rgb, 0, n_c * raw1, ctx->stream));
+                           return hoh_decode_images(ctx, s.packed, padded, s.off, n_c, width, height, s.rgb,
+                                                    static_cast<int32_t*>(s.rec));
+                       });
 }
 
 // =================================================================================================

@@ -251,12 +251,18 @@ int hoh_decode_images_s0(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_by
                          uint32_t height, const uint16_t* d_backref, uint8_t* d_rgb,
                          int32_t* d_status /* n_images*streams_per_image */);
 
-/* Host-buffer forms of the two calls above — what a host container writer / reader calls: the RGB
- * (or packed) bytes are copied to the device, coded, and the result copied back, all on the context's
- * stream; device staging lives in the context and is reused across calls.  Pass pinned buffers
+/* Host-buffer forms of the two calls above — what a host container writer / reader calls: the batch is
+ * cut into chunks of whole images that are pipelined, up to four in flight: while one chunk is copied in,
+ * earlier ones are coded (each in a child context of its own, so their kernels run concurrently) and
+ * copied out, on copy streams of the context.  Work queued on the context's stream before the call
+ * happens first.  Device staging lives in the context and is reused across calls.  Pass pinned buffers
  * (hoh_host_alloc) for full copy bandwidth.  encode: packed_host/packed_cap receive the channel
  * payloads back to back, off_host (n_streams+1 u64) their offsets, results_host (n_streams, may be
- * NULL) the per-stream results.  decode: status_host (n_streams, may be NULL). */
+ * NULL) the per-stream results; HOH_E_CAPACITY when packed_cap is too small.  decode: exact sizes, no
+ * padding needed; status_host (n_streams, may be NULL); HOH_E_ARG when off_host runs backwards or past
+ * packed_bytes between chunks (a bad range inside a chunk fails its stream's status).  On any failure
+ * of these two calls, or of the whole-tile host calls below, every copy and kernel of the call has been
+ * drained before it returns, and the context stays usable. */
 int hoh_encode_images_s0_host(hoh_ctx* ctx, const uint8_t* rgb_host, size_t n_images, uint32_t width,
                               uint32_t height, uint8_t* packed_host, size_t packed_cap, uint64_t* off_host,
                               hoh_stream_result* results_host);
