@@ -23,7 +23,7 @@ enum Slot {
     S_FREQS = 0, S_CUM, S_HEADS, S_ENCMETA, S_DECMETA, S_RESID, S_STREAMS, S_DSTREAMS, S_DRESULTS,
     S_IO_A, S_IO_B, S_IO_C, S_IO_D, S_IO_E, S_RESULTS, S_TOP, S_BP, S_HIST, S_COST, S_SUMS, S_MASKS,
     S_WIDE_TOP, S_WIDE_BP, S_MISC, S_L_MAPS, S_L_IDX, S_L_HDR, S_L_U32, S_L_STATUS, S_L_RR, S_L_RES, S_LZ_PX, S_LZ_STATE, S_LZ_SIDE, S_LZ_COUNTS, S_LZ_SLABS, S_LZ_RES, S_LZ_BONUS, S_LZ_KEYS, S_LZ_VALS, S_LZ_FLAG, S_T_NUKE, S_T_LZ, S_T_U32, S_T_P8, S_T_P9, S_T_O8, S_T_O9, S_T_R8, S_T_R9, S_T_MORE_SHAPES, S_T_LAST = S_T_NUKE + 4 * 9 - 1, S_D_TILES, S_D_PLANES, S_D_LZSYM, S_D_IDXSYM, S_D_RESID, S_D_OUT, S_D_BACKREF, S_D_MAPS,
-    S_D_STREAMS, S_D_RES_A, S_D_RES_B, S_D_TOP, S_D_BP, S_D_PSTATUS, S_L_NEED, S_L_ORDER, S_COUNT
+    S_D_STREAMS, S_D_RES_A, S_D_RES_B, S_D_TOP, S_D_BP, S_D_PSTATUS, S_L_NEED, S_L_ORDER, S_R_SLOTS, S_R_STATUS, S_COUNT
 };
 
 struct Buf {
@@ -45,7 +45,9 @@ struct hoh_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     uint64_t launches = 0;
-    uint64_t enc_key = 0, dec_key = 0;  // image shape / mode the cached scratch of the chunked walks was sized for
+    // image shape / mode (and crop size) the cached scratch of the chunked walks was sized for: hoh_encode_images,
+    // hoh_decode_images, hoh_decode_regions
+    uint64_t enc_key = 0, dec_key = 0, roi_key = 0;
     char err[512] = {0};
     Buf scratch[S_COUNT];
     cudaEvent_t ev[16][2] = {};
@@ -240,7 +242,7 @@ size_t scratch_budget(hoh_ctx* ctx) {
     return budget;
 }
 
-int new_shape(hoh_ctx* ctx, uint64_t key, bool decode);
+int new_shape(hoh_ctx* ctx, uint64_t key, uint64_t& slot);
 
 inline unsigned blocks_for(uint64_t items, unsigned per_block) { return (unsigned)((items + per_block - 1) / per_block); }
 inline unsigned grid_cap(uint64_t items, unsigned per_block, unsigned cap = 148u * 32u) {
@@ -554,8 +556,7 @@ namespace {
 // The chunked walks size their scratch from what the device has free plus what the context already holds, which
 // is only true while the held buffers have the proportions the walk wants: when the image shape or mode changes
 // between calls, the cached scratch of the previous shape is released first.
-int new_shape(hoh_ctx* ctx, uint64_t key, bool decode) {
-    uint64_t& slot = decode ? ctx->dec_key : ctx->enc_key;
+int new_shape(hoh_ctx* ctx, uint64_t key, uint64_t& slot) {
     if (slot == key) return HOH_OK;
     if (slot != 0) {
         // this context's own codec scratch and the two children the encoder forks into; NOT children 2 and 3,
@@ -1101,16 +1102,18 @@ struct PipeSlot {
 };
 
 // One host-buffer call: chunk c holds images bounds[c] .. bounds[c+1] and goes through slot c % depth.  A unit is one
-// entry of the offset table: a stream (s0 calls) or a tile (whole-tile calls).
+// entry of the offset table: a stream (s0 calls) or a tile (whole-tile calls).  Every unit has a record, except in
+// hoh_decode_regions_host, which has one status per image (recs = 1).
 struct Pipe {
     hoh_ctx* ctx;
     std::vector<size_t> bounds;
-    size_t raw1, units, rec_bytes;  // per image: bytes of pixels and units; bytes of one unit's record
+    size_t raw1, units, rec_bytes;  // per image: bytes of pixels and units; bytes of one record
+    size_t recs;                    // records per image
     size_t max_chunk = 0;           // images in the largest chunk
     int depth;
     PipeSlot slot[kPipeDepth];
     Pipe(hoh_ctx* c, std::vector<size_t> b, int max_depth, size_t raw_per_image, size_t units_per_image, size_t rec)
-        : ctx(c), bounds(std::move(b)), raw1(raw_per_image), units(units_per_image), rec_bytes(rec) {
+        : ctx(c), bounds(std::move(b)), raw1(raw_per_image), units(units_per_image), rec_bytes(rec), recs(units_per_image) {
         for (size_t k = 0; k < chunks(); k++) max_chunk = std::max(max_chunk, bounds[k + 1] - bounds[k]);
         depth = (int)std::min(chunks(), (size_t)max_depth);
     }
@@ -1190,7 +1193,7 @@ int pipe_begin(Pipe& pp, size_t packed_cap) {
         TRY(scratch_t(s.stage, S_IO_A, pp.max_chunk * pp.raw1, &s.rgb));
         TRY(scratch_t(s.stage, S_IO_B, packed_cap, &s.packed));
         TRY(scratch_t(s.stage, S_IO_C, units + 1, &s.off));
-        TRY(scratch(s.stage, S_IO_D, units * pp.rec_bytes, &s.rec));
+        TRY(scratch(s.stage, S_IO_D, pp.max_chunk * pp.recs * pp.rec_bytes, &s.rec));
         TRY(pinned_off(ctx, b, units + 1, &s.h_off));
     }
     CK(cudaEventRecord(ctx->ev_start, ctx->stream));
@@ -1273,20 +1276,45 @@ int pipe_encode(Pipe& pp, size_t dev_cap, const uint8_t* rgb_host, uint8_t* pack
     return HOH_OK;
 }
 
+// pipe_decode's copy-in hook: where a chunk's payloads come from and where they land in its staging.  This one, for the
+// whole-image calls, stages one range of packed_host per chunk, from its first unit's start to its last unit's end.
+struct RangeIn {
+    // bytes chunk c stages; HOH_E_ARG when its offsets run backwards or past packed_bytes
+    int bytes(const Pipe& pp, size_t c, const uint64_t* off_host, size_t packed_bytes, uint64_t* out) const {
+        const uint64_t lo = off_host[pp.bounds[c] * pp.units], hi = off_host[pp.bounds[c + 1] * pp.units];
+        if (hi < lo || hi > packed_bytes) return HOH_E_ARG;
+        *out = hi - lo;
+        return HOH_OK;
+    }
+    // chunk c's offset table (units of the chunk + 1 entries) rebased onto its staging
+    void rebase(const Pipe& pp, size_t c, const uint64_t* off_host, uint64_t* h_off) const {
+        const size_t u0 = pp.bounds[c] * pp.units, nu = (pp.bounds[c + 1] - pp.bounds[c]) * pp.units;
+        for (size_t i = 0; i <= nu; i++) h_off[i] = off_host[u0 + i] - off_host[u0];
+    }
+    // queues the copies of chunk c's payloads (bytes of them) into dst on the H2D copy stream
+    int copy(const Pipe& pp, size_t c, const uint8_t* packed_host, const uint64_t* off_host, uint64_t bytes,
+             uint8_t* dst) const {
+        hoh_ctx* ctx = pp.ctx;
+        CK(cudaMemcpyAsync(dst, packed_host + off_host[pp.bounds[c] * pp.units], bytes, cudaMemcpyHostToDevice, ctx->s_h2d));
+        return HOH_OK;
+    }
+};
+
 // Decodes the chunks of a host-buffer call.  code(b, n_images, packed_bytes) decodes the chunk in slot b on the slot's
 // run context: payloads in packed (packed_bytes, zero padding included), chunk-relative offsets in off, pixels to rgb,
-// per-unit status to rec.  Per chunk: rebase its offsets on the host, pad, H2D payloads and offsets, code, D2H pixels
-// and status.  Offsets that decrease from one chunk to the next or end beyond packed_bytes are HOH_E_ARG.
-template <class Code>
+// records (status) to rec.  Per chunk: rebase its offsets on the host, pad, H2D payloads (through the copy-in hook
+// `in`) and offsets, code, D2H pixels and records.  The hook's HOH_E_ARG (offsets that run backwards or past
+// packed_bytes) comes before anything is queued.
+template <class Code, class In = RangeIn>
 int pipe_decode(Pipe& pp, const uint8_t* packed_host, size_t packed_bytes, const uint64_t* off_host, uint8_t* rgb_host,
-                int32_t* status_host, Code code) {
+                int32_t* status_host, Code code, const In& in = In()) {
     hoh_ctx* ctx = pp.ctx;
     const size_t n_chunks = pp.chunks(), depth = pp.depth, units = pp.units;
+    std::vector<uint64_t> chunk_bytes(n_chunks);
     size_t max_packed = 0;
     for (size_t c = 0; c < n_chunks; c++) {
-        const uint64_t lo = off_host[pp.bounds[c] * units], hi = off_host[pp.bounds[c + 1] * units];
-        if (hi < lo || hi > packed_bytes) return HOH_E_ARG;
-        max_packed = std::max<size_t>(max_packed, hi - lo);
+        TRY(in.bytes(pp, c, off_host, packed_bytes, &chunk_bytes[c]));
+        max_packed = std::max<size_t>(max_packed, chunk_bytes[c]);
     }
     // >= 32 zero bytes behind a chunk's last payload byte (the decode input contract, hohgpu.h)
     auto padded = [](size_t bytes) { return (bytes + 47) & ~(size_t)15; };
@@ -1295,14 +1323,14 @@ int pipe_decode(Pipe& pp, const uint8_t* packed_host, size_t packed_bytes, const
     for (size_t c = 0; c < n_chunks; c++) {
         const int b = (int)(c % depth);
         const PipeSlot& s = pp.slot[b];
-        const size_t first = pp.bounds[c], n_c = pp.bounds[c + 1] - first, u0 = first * units, nu = n_c * units;
-        const uint64_t lo = off_host[u0], bytes = off_host[u0 + nu] - lo;
+        const size_t first = pp.bounds[c], n_c = pp.bounds[c + 1] - first, nu = n_c * units;
+        const uint64_t bytes = chunk_bytes[c];
         const size_t aligned = bytes & ~(size_t)15;
         if (c >= depth) CK(cudaEventSynchronize(ctx->ev_h2d[b]));  // s.h_off was read by chunk c-depth's copy
-        for (size_t i = 0; i <= nu; i++) s.h_off[i] = off_host[u0 + i] - lo;
+        in.rebase(pp, c, off_host, s.h_off);
         if (c >= depth) CK(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_comp[b], 0));  // s.packed / s.off consumed
         CK(cudaMemsetAsync(s.packed + aligned, 0, padded(bytes) - aligned, ctx->s_h2d));
-        CK(cudaMemcpyAsync(s.packed, packed_host + lo, bytes, cudaMemcpyHostToDevice, ctx->s_h2d));
+        TRY(in.copy(pp, c, packed_host, off_host, bytes, s.packed));
         CK(cudaMemcpyAsync(s.off, s.h_off, (nu + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->s_h2d));
         CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
         CK(cudaStreamWaitEvent(s.run->stream, ctx->ev_h2d[b], 0));
@@ -1312,7 +1340,8 @@ int pipe_decode(Pipe& pp, const uint8_t* packed_host, size_t packed_bytes, const
         CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_comp[b], 0));
         CK(cudaMemcpyAsync(rgb_host + first * pp.raw1, s.rgb, n_c * pp.raw1, cudaMemcpyDeviceToHost, ctx->s_d2h));
         if (status_host)
-            CK(cudaMemcpyAsync(status_host + u0, s.rec, nu * pp.rec_bytes, cudaMemcpyDeviceToHost, ctx->s_d2h));
+            CK(cudaMemcpyAsync(status_host + first * pp.recs, s.rec, n_c * pp.recs * pp.rec_bytes, cudaMemcpyDeviceToHost,
+                               ctx->s_d2h));
         CK(cudaEventRecord(ctx->ev_d2h[b], ctx->s_d2h));
     }
     CK(cudaStreamSynchronize(ctx->s_d2h));
@@ -1927,7 +1956,7 @@ int hoh_encode_images(hoh_ctx* ctx, const uint8_t* d_rgb, size_t n_images, uint3
                       4 * hoh_enc_slab_bytes(lz_side_stride(npx), 10) +
                       3 * (2 * npx * 2 + 8192) + 4096);
     }
-    TRY(new_shape(ctx, ((uint64_t)width << 40) ^ ((uint64_t)height << 16) ^ ((uint64_t)mode << 8) ^ 1u, false));
+    TRY(new_shape(ctx, ((uint64_t)width << 40) ^ ((uint64_t)height << 16) ^ ((uint64_t)mode << 8) ^ 1u, ctx->enc_key));
     const size_t budget = scratch_budget(ctx);
     size_t images_per_chunk = budget / per_image;
     if (images_per_chunk == 0) images_per_chunk = 1;
@@ -2010,6 +2039,122 @@ int hoh_encode_images(hoh_ctx* ctx, const uint8_t* d_rgb, size_t n_images, uint3
 // -------------------------------------------------------------------------------------------------
 // tile decoder, any cruncher mode (inverse of hoh_encode_images)
 // -------------------------------------------------------------------------------------------------
+} // extern "C" (reopened below)
+namespace {
+// Scratch of the tile decoder's phases for up to `ct` tiles of one shape per pass (hoh_decode_images: every tile of a
+// chunk's images; hoh_decode_regions: the slots of one shape).
+struct DecScratch {
+    uint32_t max_cells, max_side;
+    size_t per_tile;  // scratch bytes per tile in a pass
+    DTile* tiles;
+    DPlane* planes;
+    uint16_t *lz_sym, *idx_sym, *resid, *out, *backref, *maps, *top;
+    uint8_t* bp;
+    int32_t* pstatus;
+    hoh_dec_stream* streams;
+    hoh_dec_result *res_a, *res_b;
+};
+int dec_sizes(const hoh_tile_geometry& hg, const TileGeom& g, DecScratch* d) {
+    d->max_cells = (((uint32_t)hg.tile_w + 39) / 40) * (((uint32_t)hg.tile_h + 39) / 40);
+    if ((hg.tile_w + 39) / 40 > 256 || (hg.tile_h + 39) / 40 > 256) return HOH_E_UNSUPPORTED;
+    d->max_side = lz_side_stride((size_t)hg.tile_w * hg.tile_h);
+    d->per_tile = 4 * (size_t)d->max_side * 2 + 3 * (size_t)g.plane_stride * 2 * 2 + (size_t)g.plane_stride * 2 +
+                  3 * (size_t)(kCumRow * 4 + kFreqRow * 4) + 3 * (size_t)hg.tile_w * 3 + 4096;
+    return HOH_OK;
+}
+int dec_scratch(hoh_ctx* ctx, const hoh_tile_geometry& hg, const TileGeom& g, size_t ct, DecScratch* d) {
+    const uint32_t max_cells_pad = (d->max_cells + 7u) & ~7u;
+    TRY(scratch_t(ctx, S_D_TILES, ct, &d->tiles));
+    TRY(scratch_t(ctx, S_D_PLANES, ct * 3, &d->planes));
+    TRY(scratch_t(ctx, S_D_LZSYM, ct * 4 * d->max_side, &d->lz_sym));
+    TRY(scratch_t(ctx, S_D_IDXSYM, ct * 3 * max_cells_pad, &d->idx_sym));
+    TRY(scratch_t(ctx, S_D_RESID, ct * 3 * g.plane_stride, &d->resid));
+    TRY(scratch_t(ctx, S_D_OUT, ct * 3 * g.plane_stride, &d->out));
+    TRY(scratch_t(ctx, S_D_BACKREF, ct * g.plane_stride, &d->backref));
+    TRY(scratch_t(ctx, S_D_MAPS, ct * 3 * d->max_cells, &d->maps));
+    TRY(scratch_t(ctx, S_D_STREAMS, ct * 3, &d->streams));
+    TRY(scratch_t(ctx, S_D_RES_A, ct * 3, &d->res_a));
+    TRY(scratch_t(ctx, S_D_RES_B, ct * 3, &d->res_b));
+    TRY(scratch_t(ctx, S_D_TOP, ct * 3 * (size_t)hg.tile_w, &d->top));
+    TRY(scratch_t(ctx, S_D_BP, ct * 3 * (size_t)hg.tile_w, &d->bp));
+    TRY(scratch_t(ctx, S_D_PSTATUS, ct * 3, &d->pstatus));
+    return HOH_OK;
+}
+// One pass of the tile decoder over nt tiles of shape tw x th (choh.cpp:459-474).  begin() launches the phase that
+// fills d.tiles / d.streams for local tiles 0 .. nt-1, store() the one that writes their pixels out; the phases in
+// between only see local tile numbers.
+template <class Begin, class Store>
+int decode_pass(hoh_ctx* ctx, const DecScratch& d, size_t nt, int tw, int th, uint32_t plane_stride,
+                const uint8_t* d_packed, size_t packed_bytes, Begin begin, Store store) {
+    const uint32_t npx = (uint32_t)tw * th;
+    const uint32_t xt = (tw + 39) / 40, yt = (th + 39) / 40, cells = xt * yt, cells_pad = (cells + 7u) & ~7u;
+    const uint32_t side = lz_side_stride(npx);
+    TRY(begin(side));
+    for (uint32_t k = 0; k < 4; k++) {  // un_lz.hpp:100-145: the side streams follow one another
+        TRY(decode_common(ctx, d.streams, nt, d_packed, packed_bytes, d.lz_sym, d.res_a));
+        k_dt_lz_next<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(nt, k, d_packed, packed_bytes, d.res_a, side, d.tiles,
+                                                                   d.streams);
+        LAUNCHED("k_dt_lz_next");
+    }
+    k_dt_channels<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(nt, d_packed, packed_bytes, xt, yt, cells_pad, d.tiles,
+                                                                d.planes, d.streams);
+    LAUNCHED("k_dt_channels");
+    TRY(decode_common(ctx, d.streams, nt * 3, d_packed, packed_bytes, d.idx_sym, d.res_a));
+    k_dt_main<<<blocks_for(nt * 3, 128), 128, 0, ctx->stream>>>(nt * 3, cells, cells_pad, plane_stride, npx, d.res_a,
+                                                                d.idx_sym, d.planes, d.maps, d.streams);
+    LAUNCHED("k_dt_main");
+    TRY(decode_common(ctx, d.streams, nt * 3, d_packed, packed_bytes, d.resid, d.res_b));
+    k_dt_unlz<<<blocks_for(nt * 32, 128), 128, 0, ctx->stream>>>(nt, npx, plane_stride, d.lz_sym, side, d.tiles, d.backref);
+    LAUNCHED("k_dt_unlz");
+    // One thread per plane with its inputs prefetched in 8-pixel groups (tile widths that are multiples of
+    // 8: 17 ms for 5 760 planes of 256x270, 37 ms for 46 080).  Other widths take the scalar walk, whose
+    // loads sit on the pixel chain: there a half-warp per predictor-grid plane is faster while the launch is
+    // bound by the length of one plane's walk (37 vs 55 ms for 5 760 planes; crossover near 20 000).
+    const bool grouped = tw % 8 == 0 && tw >= 16 && plane_stride % 8 == 0;  // k_dt_unpredict's prefetched walk
+    const bool wide_walk = !grouped && nt * 3 <= 16384;
+    k_dt_unpredict<<<blocks_for(nt * 3, 64), 64, 0, ctx->stream>>>(nt * 3, tw, th, (int)xt, (int)yt, plane_stride,
+                                                                   d.planes, d.tiles, d.res_b, d.resid, d.maps, d.backref,
+                                                                   d.out, d.top, d.bp, d.pstatus, wide_walk ? 1u : 0u);
+    LAUNCHED("k_dt_unpredict");
+    if (wide_walk) {
+        k_dt_unpredict16<<<blocks_for(nt * 3, kUp16Planes), kUp16Planes * 16,
+                           (size_t)kUp16Planes * ((tw + 1) & ~1) * 3, ctx->stream>>>(
+            nt * 3, tw, th, (int)xt, (int)yt, plane_stride, d.planes, d.tiles, d.res_b, d.resid, d.maps, d.backref, d.out,
+            d.pstatus);
+        LAUNCHED("k_dt_unpredict16");
+    }
+    return store();
+}
+
+// Slots per tile shape of a region decode (RoiPlan, hoh_kernels.cuh) and the shapes' sub-grids.
+// Bound: a window covers pixel columns wx .. wx + crop_w - 1, and column x lies in tile column floor(x / tile_w).  For
+// integers a, b >= 0, floor((a + b) / t) - floor(a / t) <= ceil(b / t), so the window touches at most
+// ceil((crop_w - 1) / tile_w) + 1 = (crop_w + tile_w - 2) / tile_w + 1 tile columns, and no more than the x_count
+// columns of a shape's sub-grid; the same holds for rows.  k_roi_select asserts it.
+RoiPlan roi_plan(const TileGeom& g, const TileClass* cls, int n_cls, uint32_t crop_w, uint32_t crop_h) {
+    RoiPlan p;
+    memset(&p, 0, sizeof(p));
+    p.g = g;
+    p.crop_w = crop_w;
+    p.crop_h = crop_h;
+    p.n_cls = (uint32_t)n_cls;
+    const uint32_t span_x = (crop_w + g.tile_w - 2) / g.tile_w + 1, span_y = (crop_h + g.tile_h - 2) / g.tile_h + 1;
+    for (int c = 0; c < n_cls; c++) {
+        const TileSel& s = cls[c].sel;
+        p.x_first[c] = s.x_first;
+        p.x_count[c] = s.x_count;
+        p.y_first[c] = s.y_first;
+        p.y_count[c] = s.y_count;
+        p.cols[c] = std::min(s.x_count, span_x);
+        p.rows[c] = std::min(s.y_count, span_y);
+        p.first[c] = p.per_image;
+        p.per_image += p.cols[c] * p.rows[c];
+    }
+    return p;
+}
+}  // namespace
+extern "C" {
+
 int hoh_decode_images(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_bytes, const uint64_t* d_tile_off,
                       size_t n_images, uint32_t width, uint32_t height, uint8_t* d_rgb, int32_t* d_status) {
     DeviceGuard guard_(ctx);
@@ -2021,86 +2166,98 @@ int hoh_decode_images(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_bytes
     const TileGeom g = to_geom(hg);
     TileClass cls[4];
     const int n_cls = tile_classes(g, cls);
-    const uint32_t max_cells = (((uint32_t)hg.tile_w + 39) / 40) * (((uint32_t)hg.tile_h + 39) / 40);
-    if ((hg.tile_w + 39) / 40 > 256 || (hg.tile_h + 39) / 40 > 256) return HOH_E_UNSUPPORTED;
-    const uint32_t max_cells_pad = (max_cells + 7u) & ~7u;
-    const uint32_t max_side = lz_side_stride((size_t)hg.tile_w * hg.tile_h);
-    const size_t per_tile = 4 * (size_t)max_side * 2 + 3 * (size_t)g.plane_stride * 2 * 2 + (size_t)g.plane_stride * 2 +
-                            3 * (size_t)(kCumRow * 4 + kFreqRow * 4) + 3 * (size_t)hg.tile_w * 3 + 4096;
-    TRY(new_shape(ctx, ((uint64_t)width << 40) ^ ((uint64_t)height << 16) ^ 2u, true));
+    DecScratch d;
+    TRY(dec_sizes(hg, g, &d));
+    TRY(new_shape(ctx, ((uint64_t)width << 40) ^ ((uint64_t)height << 16) ^ 2u, ctx->dec_key));
     const size_t budget = scratch_budget(ctx);
-    size_t images_per_chunk = budget / (per_tile * g.tiles_per_image);
+    size_t images_per_chunk = budget / (d.per_tile * g.tiles_per_image);
     if (images_per_chunk == 0) images_per_chunk = 1;
     if (images_per_chunk > n_images) images_per_chunk = n_images;
-    const size_t ct = images_per_chunk * g.tiles_per_image;  // upper bound for any one shape's tiles in a chunk
-    DTile* tiles;
-    DPlane* planes;
-    uint16_t *lz_sym, *idx_sym, *resid, *out, *backref, *maps, *top;
-    uint8_t* bp;
-    int32_t* pstatus;
-    hoh_dec_stream* streams;
-    hoh_dec_result *res_a, *res_b;
-    TRY(scratch_t(ctx, S_D_TILES, ct, &tiles));
-    TRY(scratch_t(ctx, S_D_PLANES, ct * 3, &planes));
-    TRY(scratch_t(ctx, S_D_LZSYM, ct * 4 * max_side, &lz_sym));
-    TRY(scratch_t(ctx, S_D_IDXSYM, ct * 3 * max_cells_pad, &idx_sym));
-    TRY(scratch_t(ctx, S_D_RESID, ct * 3 * g.plane_stride, &resid));
-    TRY(scratch_t(ctx, S_D_OUT, ct * 3 * g.plane_stride, &out));
-    TRY(scratch_t(ctx, S_D_BACKREF, ct * g.plane_stride, &backref));
-    TRY(scratch_t(ctx, S_D_MAPS, ct * 3 * max_cells, &maps));
-    TRY(scratch_t(ctx, S_D_STREAMS, ct * 3, &streams));
-    TRY(scratch_t(ctx, S_D_RES_A, ct * 3, &res_a));
-    TRY(scratch_t(ctx, S_D_RES_B, ct * 3, &res_b));
-    TRY(scratch_t(ctx, S_D_TOP, ct * 3 * (size_t)hg.tile_w, &top));
-    TRY(scratch_t(ctx, S_D_BP, ct * 3 * (size_t)hg.tile_w, &bp));
-    TRY(scratch_t(ctx, S_D_PSTATUS, ct * 3, &pstatus));
+    // upper bound for any one shape's tiles in a chunk
+    TRY(dec_scratch(ctx, hg, g, images_per_chunk * g.tiles_per_image, &d));
     for (size_t img0 = 0; img0 < n_images; img0 += images_per_chunk) {
         const size_t ni = std::min(images_per_chunk, n_images - img0);
         for (int c = 0; c < n_cls; c++) {  // one pass per tile shape (choh.cpp:459-474)
             const TileSel& sel = cls[c].sel;
-            const int tw = cls[c].tw, th = cls[c].th;
-            const uint32_t npx = (uint32_t)tw * th;
-            const uint32_t xt = (tw + 39) / 40, yt = (th + 39) / 40, cells = xt * yt, cells_pad = (cells + 7u) & ~7u;
-            const uint32_t side = lz_side_stride(npx);
             const size_t nt = ni * sel.per_image;
-            k_dt_begin<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(nt, sel, img0, d_packed, packed_bytes, d_tile_off, side,
-                                                                     tiles, streams);
-            LAUNCHED("k_dt_begin");
-            for (uint32_t k = 0; k < 4; k++) {  // un_lz.hpp:100-145: the side streams follow one another
-                TRY(decode_common(ctx, streams, nt, d_packed, packed_bytes, lz_sym, res_a));
-                k_dt_lz_next<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(nt, k, d_packed, packed_bytes, res_a, side, tiles,
-                                                                           streams);
-                LAUNCHED("k_dt_lz_next");
-            }
-            k_dt_channels<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(nt, d_packed, packed_bytes, xt, yt, cells_pad, tiles,
-                                                                        planes, streams);
-            LAUNCHED("k_dt_channels");
-            TRY(decode_common(ctx, streams, nt * 3, d_packed, packed_bytes, idx_sym, res_a));
-            k_dt_main<<<blocks_for(nt * 3, 128), 128, 0, ctx->stream>>>(nt * 3, cells, cells_pad, g.plane_stride, npx, res_a,
-                                                                        idx_sym, planes, maps, streams);
-            LAUNCHED("k_dt_main");
-            TRY(decode_common(ctx, streams, nt * 3, d_packed, packed_bytes, resid, res_b));
-            k_dt_unlz<<<blocks_for(nt * 32, 128), 128, 0, ctx->stream>>>(nt, npx, g.plane_stride, lz_sym, side, tiles, backref);
-            LAUNCHED("k_dt_unlz");
-            // One thread per plane with its inputs prefetched in 8-pixel groups (tile widths that are multiples of
-            // 8: 17 ms for 5 760 planes of 256x270, 37 ms for 46 080).  Other widths take the scalar walk, whose
-            // loads sit on the pixel chain: there a half-warp per predictor-grid plane is faster while the launch is
-            // bound by the length of one plane's walk (37 vs 55 ms for 5 760 planes; crossover near 20 000).
-            const bool grouped = tw % 8 == 0 && tw >= 16 && g.plane_stride % 8 == 0;  // k_dt_unpredict's prefetched walk
-            const bool wide_walk = !grouped && nt * 3 <= 16384;
-            k_dt_unpredict<<<blocks_for(nt * 3, 64), 64, 0, ctx->stream>>>(nt * 3, tw, th, (int)xt, (int)yt, g.plane_stride,
-                                                                           planes, tiles, res_b, resid, maps, backref, out,
-                                                                           top, bp, pstatus, wide_walk ? 1u : 0u);
-            LAUNCHED("k_dt_unpredict");
-            if (wide_walk) {
-                k_dt_unpredict16<<<blocks_for(nt * 3, kUp16Planes), kUp16Planes * 16,
-                                   (size_t)kUp16Planes * ((tw + 1) & ~1) * 3, ctx->stream>>>(
-                    nt * 3, tw, th, (int)xt, (int)yt, g.plane_stride, planes, tiles, res_b, resid, maps, backref, out, pstatus);
-                LAUNCHED("k_dt_unpredict16");
-            }
-            k_dt_store<<<(unsigned)nt, 256, 0, ctx->stream>>>(sel, img0, g.plane_stride, tiles, pstatus, out, d_rgb, d_status);
-            LAUNCHED("k_dt_store");
+            TRY(decode_pass(
+                ctx, d, nt, cls[c].tw, cls[c].th, g.plane_stride, d_packed, packed_bytes,
+                [&](uint32_t side) {
+                    k_dt_begin<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(nt, sel, img0, d_packed, packed_bytes,
+                                                                             d_tile_off, side, d.tiles, d.streams);
+                    LAUNCHED("k_dt_begin");
+                    return HOH_OK;
+                },
+                [&]() {
+                    k_dt_store<<<(unsigned)nt, 256, 0, ctx->stream>>>(sel, img0, g.plane_stride, d.tiles, d.pstatus, d.out,
+                                                                      d_rgb, d_status);
+                    LAUNCHED("k_dt_store");
+                    return HOH_OK;
+                }));
         }
+    }
+    return HOH_OK;
+}
+
+// -------------------------------------------------------------------------------------------------
+// region decoder: the tiles of each image's window only
+// -------------------------------------------------------------------------------------------------
+int hoh_decode_regions(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_bytes, const uint64_t* d_tile_off,
+                       size_t n_images, uint32_t width, uint32_t height, const uint32_t* d_origin,
+                       uint32_t crop_w, uint32_t crop_h, uint8_t* d_crops, int32_t* d_status) {
+    DeviceGuard guard_(ctx);
+    if (!ctx || !d_packed || !d_tile_off || !d_origin || !d_crops || !d_status) return HOH_E_ARG;
+    if (crop_w == 0 || crop_h == 0 || crop_w > width || crop_h > height) return HOH_E_ARG;
+    if (n_images == 0) return HOH_OK;
+    if (packed_bytes < 32) return HOH_E_ARG;  // input contract (hohgpu.h)
+    hoh_tile_geometry hg;
+    TRY(hoh_tile_geometry_for(width, height, &hg));
+    const TileGeom g = to_geom(hg);
+    TileClass cls[4];
+    const int n_cls = tile_classes(g, cls);
+    const RoiPlan plan = roi_plan(g, cls, n_cls, crop_w, crop_h);
+    DecScratch d;
+    TRY(dec_sizes(hg, g, &d));
+    TRY(new_shape(ctx, ((uint64_t)width << 40) ^ ((uint64_t)height << 16) ^ ((uint64_t)crop_w << 28) ^
+                           ((uint64_t)crop_h << 4) ^ 3u,
+                  ctx->roi_key));
+    const size_t budget = scratch_budget(ctx);
+    size_t images_per_chunk = budget / (d.per_tile * plan.per_image + 8 * plan.per_image);
+    if (images_per_chunk == 0) images_per_chunk = 1;
+    if (images_per_chunk > n_images) images_per_chunk = n_images;
+    uint32_t max_cls = 0;  // slots of the largest shape: one pass's tiles per image
+    for (int c = 0; c < n_cls; c++) max_cls = std::max(max_cls, plan.cols[c] * plan.rows[c]);
+    TRY(dec_scratch(ctx, hg, g, images_per_chunk * max_cls, &d));
+    uint32_t* slots;
+    int32_t* slot_status;
+    TRY(scratch_t(ctx, S_R_SLOTS, images_per_chunk * plan.per_image, &slots));
+    TRY(scratch_t(ctx, S_R_STATUS, images_per_chunk * plan.per_image, &slot_status));
+    for (size_t img0 = 0; img0 < n_images; img0 += images_per_chunk) {
+        const size_t ni = std::min(images_per_chunk, n_images - img0);
+        k_roi_select<<<blocks_for(ni, 128), 128, 0, ctx->stream>>>(ni, img0, d_origin, plan, slots);
+        LAUNCHED("k_roi_select");
+        for (int c = 0; c < n_cls; c++) {
+            const uint32_t cls_slots = plan.cols[c] * plan.rows[c], first = plan.first[c];
+            const size_t nt = ni * cls_slots;
+            TRY(decode_pass(
+                ctx, d, nt, cls[c].tw, cls[c].th, g.plane_stride, d_packed, packed_bytes,
+                [&](uint32_t side) {
+                    k_dt_begin_roi<<<blocks_for(nt, 128), 128, 0, ctx->stream>>>(
+                        nt, cls_slots, first, plan.per_image, g.tiles_per_image, img0, d_packed, packed_bytes, d_tile_off,
+                        side, slots, d.tiles, d.streams);
+                    LAUNCHED("k_dt_begin_roi");
+                    return HOH_OK;
+                },
+                [&]() {
+                    k_dt_store_window<<<(unsigned)nt, 256, 0, ctx->stream>>>(cls_slots, first, img0, plan, g.plane_stride,
+                                                                             d_origin, slots, d.tiles, d.pstatus, d.out,
+                                                                             d_crops, slot_status);
+                    LAUNCHED("k_dt_store_window");
+                    return HOH_OK;
+                }));
+        }
+        k_roi_fold<<<blocks_for(ni, 128), 128, 0, ctx->stream>>>(ni, img0, plan, slots, slot_status, d_status);
+        LAUNCHED("k_roi_fold");
     }
     return HOH_OK;
 }
@@ -2116,9 +2273,10 @@ namespace {
 // chunks) while the copies it would hide are short (6.4 GB at 55 GB/s = 116 ms).  Two chunks: the second one's H2D and
 // the first one's D2H overlap the kernels, and the chain is paid twice, not four times; one chunk when the batch is
 // small.  The double-buffered staging (raw + packed, twice) must leave most of the device to the codec's own scratch.
-std::vector<size_t> tile_chunk_plan(size_t n_images, size_t raw_per_image) {
+// floor_bytes: the smallest chunk, in bytes of pixels.
+std::vector<size_t> tile_chunk_plan(size_t n_images, size_t raw_per_image, size_t floor_bytes = (size_t)256 << 20) {
     size_t per = (n_images + 1) / 2;
-    const size_t min_per = (256u << 20) / (raw_per_image ? raw_per_image : 1) + 1;
+    const size_t min_per = floor_bytes / (raw_per_image ? raw_per_image : 1) + 1;
     if (per < min_per) per = min_per;
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
@@ -2183,6 +2341,113 @@ int hoh_decode_images_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t pack
                            return hoh_decode_images(ctx, s.packed, padded, s.off, n_c, width, height, s.rgb,
                                                     static_cast<int32_t*>(s.rec));
                        });
+}
+
+} // extern "C" (reopened below)
+namespace {
+// pipe_decode's copy-in hook for hoh_decode_regions_host.  A run is one tile row of one image's window: tiles
+// [a, b) of the offset table, contiguous in packed_host.  Only runs are staged, back to back; every tile of a run keeps
+// its place in the run and every other tile gets an empty range at the current end of the staging, so the rebased table
+// stays ascending.  The chunk's origins follow its payloads to the slot's device copy of them.
+struct RegionIn {
+    std::vector<std::vector<std::pair<size_t, size_t>>> runs;  // per image, ascending
+    const uint32_t* origin_host;
+    uint32_t* d_origin[kPipeDepth];
+    // tile rows the window at (wx, wy) of image i touches; none for a window that does not lie inside the image
+    RegionIn(const hoh_tile_geometry& hg, size_t n_images, const uint32_t* origin, uint32_t crop_w, uint32_t crop_h)
+        : runs(n_images), origin_host(origin) {
+        for (size_t i = 0; i < n_images; i++) {
+            const uint64_t wx = origin[2 * i], wy = origin[2 * i + 1];
+            if (wx + crop_w > hg.width || wy + crop_h > hg.height) continue;
+            const size_t tx0 = wx / hg.tile_w, tx1 = (wx + crop_w - 1) / hg.tile_w;
+            for (size_t ty = wy / hg.tile_h; ty <= (wy + crop_h - 1) / hg.tile_h; ty++) {
+                const size_t row = i * hg.tiles_per_image + ty * hg.x_tiles;
+                runs[i].emplace_back(row + tx0, row + tx1 + 1);
+            }
+        }
+    }
+    int bytes(const Pipe& pp, size_t c, const uint64_t* off_host, size_t packed_bytes, uint64_t* out) const {
+        uint64_t sum = 0;
+        for (size_t i = pp.bounds[c]; i < pp.bounds[c + 1]; i++)
+            for (const auto& r : runs[i]) {
+                for (size_t t = r.first; t < r.second; t++)
+                    if (off_host[t + 1] < off_host[t]) return HOH_E_ARG;
+                if (off_host[r.second] > packed_bytes) return HOH_E_ARG;
+                sum += off_host[r.second] - off_host[r.first];
+            }
+        *out = sum;
+        return HOH_OK;
+    }
+    void rebase(const Pipe& pp, size_t c, const uint64_t* off_host, uint64_t* h_off) const {
+        const size_t u0 = pp.bounds[c] * pp.units, u1 = pp.bounds[c + 1] * pp.units;
+        size_t u = u0;
+        uint64_t at = 0;
+        for (size_t i = pp.bounds[c]; i < pp.bounds[c + 1]; i++)
+            for (const auto& r : runs[i]) {
+                for (; u < r.first; u++) h_off[u - u0] = at;
+                for (; u < r.second; u++) h_off[u - u0] = at + off_host[u] - off_host[r.first];
+                at += off_host[r.second] - off_host[r.first];
+            }
+        for (; u <= u1; u++) h_off[u - u0] = at;
+    }
+    // one copy per run, straight from the caller's buffer (tools/bench_regions.py measures it against a host-side
+    // gather into pinned staging followed by one copy)
+    int copy(const Pipe& pp, size_t c, const uint8_t* packed_host, const uint64_t* off_host, uint64_t,
+             uint8_t* dst) const {
+        hoh_ctx* ctx = pp.ctx;
+        uint64_t at = 0;
+        for (size_t i = pp.bounds[c]; i < pp.bounds[c + 1]; i++)
+            for (const auto& r : runs[i]) {
+                const uint64_t len = off_host[r.second] - off_host[r.first];
+                CK(cudaMemcpyAsync(dst + at, packed_host + off_host[r.first], len, cudaMemcpyHostToDevice, ctx->s_h2d));
+                at += len;
+            }
+        const size_t n_c = pp.bounds[c + 1] - pp.bounds[c];
+        CK(cudaMemcpyAsync(d_origin[c % pp.depth], origin_host + 2 * pp.bounds[c], n_c * 2 * sizeof(uint32_t),
+                           cudaMemcpyHostToDevice, ctx->s_h2d));
+        return HOH_OK;
+    }
+};
+}  // namespace
+extern "C" {
+
+int hoh_decode_regions_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t packed_bytes,
+                            const uint64_t* tile_off_host, size_t n_images, uint32_t width, uint32_t height,
+                            const uint32_t* origin_host, uint32_t crop_w, uint32_t crop_h,
+                            uint8_t* crops_host, int32_t* status_host) {
+    DeviceGuard guard_(ctx);
+    if (!ctx || !packed_host || !tile_off_host || !origin_host || !crops_host || !status_host) return HOH_E_ARG;
+    if (crop_w == 0 || crop_h == 0 || crop_w > width || crop_h > height) return HOH_E_ARG;
+    if (n_images == 0) return HOH_OK;
+    hoh_tile_geometry hg;
+    TRY(hoh_tile_geometry_for(width, height, &hg));
+    const TileGeom g = to_geom(hg);
+    TileClass cls[4];
+    const int n_cls = tile_classes(g, cls);
+    const RoiPlan plan = roi_plan(g, cls, n_cls, crop_w, crop_h);
+    size_t touched = 0;  // bytes of pixels of the tiles an image's slots decode: what a chunk is planned by
+    for (int c = 0; c < n_cls; c++) touched += (size_t)plan.cols[c] * plan.rows[c] * cls[c].tw * cls[c].th * 3;
+    // HOH_PIPE_CHUNK_KB lowers the floor (tests: two chunks of a small batch)
+    const size_t floor_bytes = getenv("HOH_PIPE_CHUNK_KB") ? std::min(pipe_chunk_floor(), (size_t)256 << 20) : (size_t)256 << 20;
+    const size_t crop1 = (size_t)crop_w * crop_h * 3;
+    Pipe pp(ctx, tile_chunk_plan(n_images, touched, floor_bytes), 2, crop1, hg.tiles_per_image, sizeof(int32_t));
+    pp.recs = 1;
+    RegionIn in(hg, n_images, origin_host, crop_w, crop_h);
+    for (int b = 0; b < pp.depth; b++) {  // decoded on ctx itself, staging out of new_shape's reach (hoh_ctx::child)
+        pp.slot[b].run = ctx;
+        TRY(child_of(ctx, 2 + b, &pp.slot[b].stage));
+        TRY(scratch_t(pp.slot[b].stage, S_IO_E, pp.max_chunk * 2, &in.d_origin[b]));
+    }
+    return pipe_decode(
+        pp, packed_host, packed_bytes, tile_off_host, crops_host, status_host,
+        [&](int b, size_t n_c, size_t padded) {
+            const PipeSlot& s = pp.slot[b];
+            // a failing tile or a bad window leaves its pixels untouched: make "untouched" mean zero
+            CK(cudaMemsetAsync(s.rgb, 0, n_c * crop1, ctx->stream));
+            return hoh_decode_regions(ctx, s.packed, padded, s.off, n_c, width, height, in.d_origin[b], crop_w, crop_h,
+                                      s.rgb, static_cast<int32_t*>(s.rec));
+        },
+        in);
 }
 
 // =================================================================================================

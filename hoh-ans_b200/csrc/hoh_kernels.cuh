@@ -14,6 +14,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cassert>
 #include <type_traits>
 
 #include "../../include/hohgpu.h"
@@ -4556,21 +4557,15 @@ struct DPlane {
     uint16_t masks[16];
 };
 
-// tile header: 00 00 | colour mode | LZ tag
-__global__ void k_dt_begin(uint64_t n_tiles, TileSel sel, uint64_t first_image, const uint8_t* __restrict__ packed,
-                           uint64_t packed_bytes, const uint64_t* __restrict__ tile_off, uint32_t side_stride,
-                           DTile* __restrict__ tiles, hoh_dec_stream* __restrict__ streams) {
-    const uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
-    if (t >= n_tiles) return;
-    const ByteView b{packed, packed_bytes};
-    uint64_t image;
-    uint32_t in_image, x0, y0, tw, th;
-    sel_tile(sel, t, image, in_image, x0, y0, tw, th);
-    const uint64_t gt = (first_image + image) * sel.g.tiles_per_image + in_image;  // the tile's index in the batch
-    const uint64_t off = tile_off[gt];
+// tile header: 00 00 | colour mode | LZ tag.  Local tile t's bytes are [off, end); status != 0 makes it a tile that
+// decodes nothing (every later phase skips a tile or plane whose status is set).
+__device__ __forceinline__ void dt_begin_tile(uint64_t t, uint64_t off, uint64_t end, int32_t status, ByteView b,
+                                              uint32_t side_stride, DTile* __restrict__ tiles,
+                                              hoh_dec_stream* __restrict__ streams) {
+    const uint64_t packed_bytes = b.size;
     DTile d;
-    d.end = tile_off[gt + 1];
-    d.status = HOH_S_OK;
+    d.end = end;
+    d.status = status;
     d.colour_mode = b[off + 2];
     // 1x1 sub-tiles (choh.cpp:112-116), a colour mode this library emits, the LZ tag find_lz_rgb writes (lz.hpp:100)
     if (b[off] != 0 || b[off + 1] != 0 || (d.colour_mode != 128u && d.colour_mode != 2u) || b[off + 3] != 0x03 ||
@@ -4587,6 +4582,19 @@ __global__ void k_dt_begin(uint64_t n_tiles, TileSel sel, uint64_t first_image, 
     st.sym_cap = d.status ? 0u : side_stride;
     st.flags = HOH_FIX_DECODER;
     streams[t] = st;
+}
+
+__global__ void k_dt_begin(uint64_t n_tiles, TileSel sel, uint64_t first_image, const uint8_t* __restrict__ packed,
+                           uint64_t packed_bytes, const uint64_t* __restrict__ tile_off, uint32_t side_stride,
+                           DTile* __restrict__ tiles, hoh_dec_stream* __restrict__ streams) {
+    const uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (t >= n_tiles) return;
+    uint64_t image;
+    uint32_t in_image, x0, y0, tw, th;
+    sel_tile(sel, t, image, in_image, x0, y0, tw, th);
+    const uint64_t gt = (first_image + image) * sel.g.tiles_per_image + in_image;  // the tile's index in the batch
+    dt_begin_tile(t, tile_off[gt], tile_off[gt + 1], HOH_S_OK, ByteView{packed, packed_bytes}, side_stride, tiles,
+                  streams);
 }
 
 // after LZ side stream k: advance, describe stream k + 1.  The fourth stream exists only for seek windows wider
@@ -5187,6 +5195,134 @@ __global__ void __launch_bounds__(256) k_dt_store(TileSel sel, uint64_t first_im
         o[0] = (uint8_t)(sub_green ? (b[i] + gr - 256u) & 255u : b[i]);
         o[2] = (uint8_t)(sub_green ? (c[i] + gr - 256u) & 255u : c[i]);
     }
+}
+
+// -------------------------------------------------------------------------------------------------
+// Region decode (hoh_decode_regions): the crop_w x crop_h window of every image; only the tiles a window touches go
+// through the phases above.  Each image gets the same number of SLOTS per tile shape, fixed on the host from the crop
+// size, so no launch size depends on the windows (no device-to-host copy).  Slot k of shape c of image i is entry
+// i * per_image + first[c] + k of the slot list: the index (in its image) of the tile it decodes, or kRoiIdle (the
+// window touches fewer tiles of the shape than it has slots), or kRoiBadWindow (the window does not lie inside the
+// image: every slot of the image).  A pass over shape c runs cols[c] * rows[c] slots per image through
+// k_dt_begin_roi, the unchanged phases and k_dt_store_window; local tile lt is slot lt % (cols * rows) of image
+// lt / (cols * rows).
+// -------------------------------------------------------------------------------------------------
+constexpr uint32_t kRoiIdle = 0xffffffffu, kRoiBadWindow = 0xfffffffeu;
+
+struct RoiPlan {
+    TileGeom g;
+    uint32_t crop_w, crop_h, n_cls;
+    uint32_t per_image;                                       // slots of one image, all shapes
+    uint32_t x_first[4], x_count[4], y_first[4], y_count[4];  // shape c's sub-grid of the tile grid (TileSel)
+    uint32_t cols[4], rows[4], first[4];                      // shape c: cols x rows slots from slot first[c]
+};
+
+// One thread per image: checks the window and lists, per shape, the touched part of the shape's sub-grid row-major.
+__global__ void k_roi_select(uint64_t n_images, uint64_t first_image, const uint32_t* __restrict__ origin, RoiPlan p,
+                             uint32_t* __restrict__ slots) {
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= n_images) return;
+    const uint32_t wx = origin[2 * (first_image + i)], wy = origin[2 * (first_image + i) + 1];
+    const bool inside = (uint64_t)wx + p.crop_w <= p.g.width && (uint64_t)wy + p.crop_h <= p.g.height;
+    uint32_t* s = slots + i * p.per_image;
+    // x lies in tile column x / tile_w (only the last column is narrower, and width <= x_tiles * tile_w)
+    const uint32_t gx0 = inside ? wx / p.g.tile_w : 0u, gx1 = inside ? (wx + p.crop_w - 1u) / p.g.tile_w : 0u;
+    const uint32_t gy0 = inside ? wy / p.g.tile_h : 0u, gy1 = inside ? (wy + p.crop_h - 1u) / p.g.tile_h : 0u;
+    for (uint32_t c = 0; c < p.n_cls; c++) {
+        const uint32_t n_slots = p.cols[c] * p.rows[c];
+        const uint32_t cx0 = max(gx0, p.x_first[c]), cx1 = min(gx1, p.x_first[c] + p.x_count[c] - 1u);
+        const uint32_t cy0 = max(gy0, p.y_first[c]), cy1 = min(gy1, p.y_first[c] + p.y_count[c] - 1u);
+        const uint32_t nx = inside && cx1 >= cx0 ? cx1 - cx0 + 1u : 0u, ny = inside && cy1 >= cy0 ? cy1 - cy0 + 1u : 0u;
+        assert(nx <= p.cols[c] && ny <= p.rows[c]);  // the bound roi_plan proves
+        for (uint32_t k = 0; k < n_slots; k++)
+            s[p.first[c] + k] = !inside ? kRoiBadWindow
+                              : k < nx * ny ? (cy0 + k / nx) * p.g.x_tiles + cx0 + k % nx
+                                            : kRoiIdle;
+    }
+}
+
+// k_dt_begin for the slots of one shape (cls_slots = cols * rows of it).  An idle or bad-window slot becomes a tile
+// with a status whose streams point at the zero padding at the end of the input (in range, and no tile's bytes):
+// every later phase skips it as it skips a damaged tile, so the bytes of untouched tiles never decide anything.
+__global__ void k_dt_begin_roi(uint64_t n_tiles, uint32_t cls_slots, uint32_t first, uint32_t per_image,
+                               uint32_t tiles_per_image, uint64_t first_image, const uint8_t* __restrict__ packed,
+                               uint64_t packed_bytes, const uint64_t* __restrict__ tile_off, uint32_t side_stride,
+                               const uint32_t* __restrict__ slots, DTile* __restrict__ tiles,
+                               hoh_dec_stream* __restrict__ streams) {
+    const uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (t >= n_tiles) return;
+    const uint64_t image = t / cls_slots;
+    const uint32_t e = slots[image * per_image + first + t % cls_slots];
+    const ByteView b{packed, packed_bytes};
+    if (e >= kRoiBadWindow) {
+        dt_begin_tile(t, packed_bytes - 32u, packed_bytes - 32u, HOH_S_BAD_WINDOW, b, side_stride, tiles, streams);
+        return;
+    }
+    const uint64_t gt = (first_image + image) * tiles_per_image + e;
+    dt_begin_tile(t, tile_off[gt], tile_off[gt + 1], HOH_S_OK, b, side_stride, tiles, streams);
+}
+
+// k_dt_store for the slots of one shape: tile ∩ window goes to the image's dense crop at (x - wx, y - wy), and the
+// slot's status to slot_status (idle and bad-window slots write nothing).
+__global__ void __launch_bounds__(256) k_dt_store_window(uint32_t cls_slots, uint32_t first, uint64_t first_image,
+                                                         RoiPlan p, uint32_t plane_stride,
+                                                         const uint32_t* __restrict__ origin,
+                                                         const uint32_t* __restrict__ slots,
+                                                         const DTile* __restrict__ tiles,
+                                                         const int32_t* __restrict__ plane_status,
+                                                         const uint16_t* __restrict__ planes,
+                                                         uint8_t* __restrict__ crops, int32_t* __restrict__ slot_status) {
+    const uint64_t lt = blockIdx.x;
+    const uint64_t image = lt / cls_slots;
+    const uint64_t at = image * p.per_image + first + lt % cls_slots;
+    const uint32_t e = slots[at];
+    if (e >= kRoiBadWindow) return;
+    int32_t st = tiles[lt].status;
+    for (int c = 0; c < 3; c++) st = st ? st : plane_status[lt * 3u + c];
+    if (threadIdx.x == 0) slot_status[at] = st;
+    if (st) return;
+    uint32_t x0, y0, tw, th;
+    tile_rect(p.g, e, x0, y0, tw, th);
+    const uint32_t wx = origin[2 * (first_image + image)], wy = origin[2 * (first_image + image) + 1];
+    const uint32_t ix0 = max(x0, wx), ix1 = min(x0 + tw, wx + p.crop_w);
+    const uint32_t iy0 = max(y0, wy), iy1 = min(y0 + th, wy + p.crop_h);
+    if (ix1 <= ix0 || iy1 <= iy0) return;  // never for a touched tile
+    const uint32_t nw = ix1 - ix0;
+    uint8_t* crop = crops + (first_image + image) * (uint64_t)p.crop_w * p.crop_h * 3u;
+    const uint16_t* a = planes + (lt * 3u) * (uint64_t)plane_stride;
+    const uint16_t* b = a + plane_stride;
+    const uint16_t* c = b + plane_stride;
+    const bool sub_green = tiles[lt].colour_mode == 128u;
+    for (uint32_t i = threadIdx.x; i < nw * (iy1 - iy0); i += blockDim.x) {
+        const uint32_t x = ix0 + i % nw, y = iy0 + i / nw;
+        const uint32_t q = (y - y0) * tw + (x - x0);
+        uint8_t* o = crop + ((uint64_t)(y - wy) * p.crop_w + (x - wx)) * 3u;
+        const uint32_t gr = a[q];
+        o[1] = (uint8_t)gr;
+        o[0] = (uint8_t)(sub_green ? (b[q] + gr - 256u) & 255u : b[q]);
+        o[2] = (uint8_t)(sub_green ? (c[q] + gr - 256u) & 255u : c[q]);
+    }
+}
+
+// One thread per image: HOH_S_BAD_WINDOW, else the status of the failing touched tile with the lowest index, else 0.
+__global__ void k_roi_fold(uint64_t n_images, uint64_t first_image, RoiPlan p, const uint32_t* __restrict__ slots,
+                           const int32_t* __restrict__ slot_status, int32_t* __restrict__ status) {
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= n_images) return;
+    const uint32_t* s = slots + i * p.per_image;
+    const int32_t* ss = slot_status + i * p.per_image;
+    int32_t st = HOH_S_OK;
+    uint32_t lowest = kRoiIdle;
+    if (s[0] == kRoiBadWindow) {
+        st = HOH_S_BAD_WINDOW;
+    } else {
+        for (uint32_t k = 0; k < p.per_image; k++)
+            if (s[k] != kRoiIdle && ss[k] != HOH_S_OK && s[k] < lowest) {
+                lowest = s[k];
+                st = ss[k];
+            }
+    }
+    status[first_image + i] = st;
 }
 
 // -------------------------------------------------------------------------------------------------

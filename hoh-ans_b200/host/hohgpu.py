@@ -120,6 +120,8 @@ SIGNATURES = {
     "hoh_decode_images": (_int, [_vp, _vp, _sz, _vp, _sz, _u32, _u32, _vp, _vp]),
     "hoh_encode_images_host": (_int, [_vp, _vp, _sz, _u32, _u32, _int, C.c_uint, _vp, _sz, _vp, _vp]),
     "hoh_decode_images_host": (_int, [_vp, _vp, _sz, _vp, _sz, _u32, _u32, _vp, _vp]),
+    "hoh_decode_regions": (_int, [_vp, _vp, _sz, _vp, _sz, _u32, _u32, _vp, _u32, _u32, _vp, _vp]),
+    "hoh_decode_regions_host": (_int, [_vp, _vp, _sz, _vp, _sz, _u32, _u32, _vp, _u32, _u32, _vp, _vp]),
     "hoh_find_lz_stride": (_sz, [_int, _int]),
     "hoh_find_lz_rgb_batch": (_int, [_vp, _vp, _sz, _int, _int, _int, C.c_uint, _vp, _vp, _vp, _sz, _vp, _vp]),
     "hoh_find_lz_images": (_int, [_vp, _vp, _sz, _u32, _u32, _int, C.c_uint, _vp, _vp, _vp, _sz, _vp, _vp]),
@@ -645,6 +647,44 @@ class HohGpu:
         self._ck(self.lib.hoh_decode_images_host(self.ctx, _ptr(packed), packed.size, _ptr(off), n_images, width, height,
                                                  _ptr(rgb), _ptr(st)), "hoh_decode_images_host")
         return rgb, st
+
+    def decode_regions(self, tiles, n_images, width, height, origins, crop_w, crop_h, fill=0):
+        """hoh_decode_regions: list of tile byte strings (n_images * tiles_per_image), origins (n_images x 2: x, y of
+        each window) -> (crops u8 (n_images, crop_h, crop_w, 3), status per image).  fill: the byte the crops hold
+        before the call (what a failing tile leaves)."""
+        off = np.zeros(len(tiles) + 1, np.uint64)
+        off[1:] = np.cumsum([len(t) for t in tiles])
+        blob = np.frombuffer(b"".join(tiles) + bytes(64), np.uint8)
+        org = np.ascontiguousarray(origins, dtype=np.uint32).reshape(n_images, 2)
+        crop_bytes = n_images * crop_w * crop_h * 3
+        d_packed = self.alloc(blob.nbytes).upload(blob)
+        d_off = self.alloc(off.nbytes).upload(off)
+        d_org = self.alloc(max(org.nbytes, 8)).upload(org)
+        d_crops = self.alloc(max(crop_bytes, 1))
+        self._ck(self.lib.hoh_dev_memset(self.ctx, d_crops.ptr, fill, max(crop_bytes, 1)), "hoh_dev_memset")
+        d_st = self.alloc(max(n_images, 1) * 4)
+        try:
+            self._ck(self.lib.hoh_decode_regions(self.ctx, d_packed.ptr, blob.nbytes, d_off.ptr, n_images, width, height,
+                                                 d_org.ptr, crop_w, crop_h, d_crops.ptr, d_st.ptr), "hoh_decode_regions")
+            crops = d_crops.download(np.uint8, crop_bytes)
+            st = d_st.download(np.int32, n_images)
+        finally:
+            for b in (d_packed, d_off, d_org, d_crops, d_st):
+                b.free()
+        return crops.reshape(n_images, crop_h, crop_w, 3), st
+
+    def decode_regions_host(self, packed, off, n_images, width, height, origins, crop_w, crop_h):
+        """hoh_decode_regions_host: exact-size host buffers and origins (n_images x 2) -> (crops (n_images, crop_h,
+        crop_w, 3), status per image).  Only the touched tiles' bytes are copied to the device."""
+        packed = np.ascontiguousarray(packed, dtype=np.uint8)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        org = np.ascontiguousarray(origins, dtype=np.uint32).reshape(n_images, 2)
+        crops = self.host_alloc(n_images * crop_w * crop_h * 3)
+        st = np.zeros(n_images, np.int32)
+        self._ck(self.lib.hoh_decode_regions_host(self.ctx, _ptr(packed), packed.size, _ptr(off), n_images, width, height,
+                                                  _ptr(org), crop_w, crop_h, _ptr(crops), _ptr(st)),
+                 "hoh_decode_regions_host")
+        return crops.reshape(n_images, crop_h, crop_w, 3), st
 
     def layer_encode_batch(self, planes, n_planes, w, h, depth, mode, nuke=None, planes_per_map=1, flags=0):
         """layer_encode.hpp:11 for n_planes planes of the same shape -> list of (payload bytes, status, kept slot).

@@ -374,6 +374,30 @@ int hoh_encode_images_host(hoh_ctx* ctx, const uint8_t* rgb_host, size_t n_image
 int hoh_decode_images_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t packed_bytes, const uint64_t* tile_off_host,
                            size_t n_images, uint32_t width, uint32_t height, uint8_t* rgb_host, int32_t* status_host);
 
+#define HOH_S_BAD_WINDOW 8  /* decode_regions: the window does not lie inside the image */
+
+/* Region decode (random access into tiled images): the crop_w x crop_h window at (origin[2i], origin[2i+1]) of image
+ * i, for every image of a batch that hoh_encode_images (or stock choh) wrote.  Only the tiles the window touches are
+ * decoded.  d_crops: n_images * crop_h * crop_w * 3 bytes, dense (crop i at i * crop_h * crop_w * 3, row-major RGB8).
+ * d_status[i] (n_images entries) is HOH_S_OK when every tile the window touches decoded.  Otherwise it is the status
+ * of the failing touched tile with the lowest tile index; that tile's part of the crop is left untouched, as in
+ * hoh_decode_images.  A window that does not lie inside its image gets HOH_S_BAD_WINDOW and its crop is untouched.
+ * The bytes of tiles the window does not touch are never decoded: they may be anything, as long as d_tile_off stays
+ * ascending.  Input contract as for hoh_decode_images (32 zero bytes of padding).  crop_w == 0, crop_h == 0,
+ * crop_w > width or crop_h > height is HOH_E_ARG; the origins are device memory, so a window that does not fit is
+ * reported per image. */
+int hoh_decode_regions(hoh_ctx* ctx, const uint8_t* d_packed, size_t packed_bytes, const uint64_t* d_tile_off,
+                       size_t n_images, uint32_t width, uint32_t height, const uint32_t* d_origin,
+                       uint32_t crop_w, uint32_t crop_h, uint8_t* d_crops, int32_t* d_status);
+/* Host-buffer form, pipelined like hoh_decode_images_host.  Exact sizes, no padding.  Only the byte ranges of touched
+ * tiles cross PCIe (one copy per touched tile row of each window).  Pixels of a failing tile, and the crop of a bad
+ * window, are zero.  HOH_E_ARG when the offsets of a touched tile row run backwards or past packed_bytes.  Drains on
+ * every failure, like the other host calls. */
+int hoh_decode_regions_host(hoh_ctx* ctx, const uint8_t* packed_host, size_t packed_bytes,
+                            const uint64_t* tile_off_host, size_t n_images, uint32_t width, uint32_t height,
+                            const uint32_t* origin_host, uint32_t crop_w, uint32_t crop_h,
+                            uint8_t* crops_host, int32_t* status_host);
+
 /* ------------------------------------------------------------------------------------------ */
 /* (v) LZ match finder — find_lz_rgb lz.hpp:6-145 (SURVEY 8(f) row 1) over N tiles                 */
 /* ------------------------------------------------------------------------------------------ */

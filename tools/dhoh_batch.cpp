@@ -9,7 +9,10 @@
 //
 //   dhoh_batch infile.hoh outfile.rgb                    the reference tool's command line (dhoh.cpp:306-318)
 //   dhoh_batch --batch outdir in1.hoh [in2.hoh ...]      many files in one GPU call per image size -> outdir/<name>.rgb
-//   option: --device N
+//   options: --device N
+//            --crop X Y W H   write only the W x H window at (X, Y) of every file (W * H * 3 bytes of RGB); only the
+//                             tiles the window touches are read and decoded (hoh_decode_regions_host).  A window that
+//                             does not lie inside an image is a CLI error (exit 1).
 // Exit codes follow dhoh.cpp:283-295: 0 ok, 1 CLI, 2 I/O, 3 unexpected end of file / no GPU, 4 incorrect bitstream,
 // 5 not implemented.
 #include <cerrno>
@@ -125,15 +128,33 @@ std::string stem_of(const std::string& path) {
 }  // namespace
 
 int main(int argc, char** argv) {
-    bool batch = false;
+    bool batch = false, crop = false;
     int device = 0;
+    uint32_t cx = 0, cy = 0, cw = 0, ch = 0;
     std::vector<std::string> pos;
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
         if (a == "--batch") batch = true;
         else if (a == "--device" && i + 1 < argc) device = std::atoi(argv[++i]);
-        else if (a == "--help" || a == "-h") {
-            std::printf("usage: dhoh_batch infile.hoh outfile.rgb\n       dhoh_batch --batch outdir in1.hoh [in2.hoh ...]\n");
+        else if (a == "--crop" && i + 4 < argc) {
+            crop = true;
+            uint32_t* v[4] = {&cx, &cy, &cw, &ch};
+            for (int k = 0; k < 4; k++) {
+                char* end = nullptr;
+                const long x = std::strtol(argv[++i], &end, 10);
+                if (!end || *end || x < 0 || x > 0x7fffffffL) {
+                    std::fprintf(stderr, "dhoh_batch: --crop takes four non-negative integers X Y W H\n");
+                    return 1;
+                }
+                *v[k] = (uint32_t)x;
+            }
+            if (cw == 0 || ch == 0) {
+                std::fprintf(stderr, "dhoh_batch: --crop: the window must not be empty\n");
+                return 1;
+            }
+        } else if (a == "--help" || a == "-h") {
+            std::printf("usage: dhoh_batch [--crop X Y W H] infile.hoh outfile.rgb\n"
+                        "       dhoh_batch [--crop X Y W H] --batch outdir in1.hoh [in2.hoh ...]\n");
             return 0;
         } else pos.push_back(a);
     }
@@ -158,6 +179,11 @@ int main(int argc, char** argv) {
     for (size_t i = 0; i < files.size(); i++) {
         if (!read_file(files[i].in, files[i].bytes)) return 2;
         if (int rc = parse_container(files[i])) return rc;
+        if (crop && ((uint64_t)cx + cw > files[i].width || (uint64_t)cy + ch > files[i].height)) {
+            std::fprintf(stderr, "dhoh_batch: --crop %u %u %u %u does not lie inside %s (%ux%u)\n", cx, cy, cw, ch,
+                         files[i].in.c_str(), files[i].width, files[i].height);
+            return 1;
+        }
         by_size[{files[i].width, files[i].height}].push_back(i);
     }
     hoh_ctx* ctx = nullptr;
@@ -172,7 +198,8 @@ int main(int argc, char** argv) {
         const std::vector<size_t>& idx = group.second;
         hoh_tile_geometry g;
         hoh_tile_geometry_for(w, h, &g);
-        const size_t n = idx.size(), raw1 = (size_t)w * h * 3, n_tiles = n * g.tiles_per_image;
+        const size_t n = idx.size(), n_tiles = n * g.tiles_per_image;
+        const size_t raw1 = crop ? (size_t)cw * ch * 3 : (size_t)w * h * 3;  // bytes written per file
         size_t total = 0;
         for (size_t i : idx) total += files[i].tile_begin.back() - files[i].tile_begin.front();
         uint8_t *packed = nullptr, *rgb = nullptr;
@@ -191,14 +218,26 @@ int main(int argc, char** argv) {
             at += len;
         }
         off[t] = at;
-        st = hoh_decode_images_host(ctx, packed, total, off.data(), n, w, h, rgb, status.data());
+        if (crop) {  // one status per file: its failing touched tile with the lowest index
+            std::vector<uint32_t> origin(2 * n);
+            for (size_t k = 0; k < n; k++) origin[2 * k] = cx, origin[2 * k + 1] = cy;
+            st = hoh_decode_regions_host(ctx, packed, total, off.data(), n, w, h, origin.data(), cw, ch, rgb, status.data());
+        } else {
+            st = hoh_decode_images_host(ctx, packed, total, off.data(), n, w, h, rgb, status.data());
+        }
         if (st != HOH_OK) {
-            std::fprintf(stderr, "dhoh_batch: hoh_decode_images_host: %s (%s)\n", hoh_strerror(st), hoh_last_cuda_error(ctx));
+            std::fprintf(stderr, "dhoh_batch: %s: %s (%s)\n", crop ? "hoh_decode_regions_host" : "hoh_decode_images_host",
+                         hoh_strerror(st), hoh_last_cuda_error(ctx));
             return 3;
         }
         for (size_t k = 0; k < n; k++) {
             const Parsed& p = files[idx[k]];
-            for (size_t j = 0; j < g.tiles_per_image; j++)
+            if (crop && status[k] != HOH_S_OK) {
+                std::fprintf(stderr, "dhoh_batch: %s: a tile of the window cannot be decoded (stream status %d)\n",
+                             p.in.c_str(), status[k]);
+                rc = 4;
+            }
+            for (size_t j = 0; j < (crop ? 0 : g.tiles_per_image); j++)
                 if (status[k * g.tiles_per_image + j] != HOH_S_OK) {
                     std::fprintf(stderr, "dhoh_batch: %s tile %zu cannot be decoded (stream status %d%s)\n", p.in.c_str(), j,
                                  status[k * g.tiles_per_image + j],
