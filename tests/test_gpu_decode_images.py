@@ -167,8 +167,9 @@ def test_decoder_survives_random_damage():
 
 
 def test_roundtrip_many_small_tiles():
-    """6 000 tiles = 18 000 planes in one call: above the plane count at which the decoder switches from the
-    half-warp un-prediction walk to one thread per plane."""
+    """6 000 tiles = 18 000 planes in one call.  The tiles are 64 wide, a multiple of 8, so every plane takes the
+    grouped un-prediction walk whatever the plane count; the one-thread-per-plane walk of other widths above 16 384
+    planes is tested in test_gpu_decode_crafted.py."""
     g = gpu_lib.gpu()
     rng = np.random.default_rng(8)
     w, h, n = 64, 48, 6000

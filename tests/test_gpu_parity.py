@@ -64,7 +64,7 @@ def test_encode_entropy_golden_vectors():
 
 
 def test_encode_entropy_batch_random_streams_vs_oracle():
-    """Ragged batch: ranges 1..512, prob_bits 8..19, empty / single-symbol / stored-mode streams."""
+    """Ragged batch: ranges 1..512, prob_bits 1..19, empty / single-symbol / stored-mode streams."""
     g = gpu_lib.gpu()
     rng = np.random.default_rng(11)
     syms, ranges, pbs, want = [], [], [], []
@@ -80,8 +80,20 @@ def test_encode_entropy_batch_random_streams_vs_oracle():
         ranges.append(rangev)
         pbs.append(pb)
         want.append((w, st))
+    # prob_bits 1..7 (the C-ABI takes 1..19), ranges up to 2^prob_bits; drawn after the streams above so that
+    # those stay as they were
+    low = np.random.default_rng(12)
+    first_low = len(syms)
+    for pb in range(1, 8):
+        for rangev in sorted({1, 2, (1 << pb) // 2 + 1, 1 << pb}):
+            for kind in range(6):
+                s = _symbols(low, kind, int(low.choice([1, 7, 64, 1000, 20000])), rangev)
+                syms.append(s)
+                ranges.append(rangev)
+                pbs.append(pb)
+                want.append(ol.orc_encode_entropy(s, rangev, pb))
     got = g.encode_entropy_batch(syms, ranges, pbs)
-    n_ok = n_stored = 0
+    n_ok = n_stored = n_low_coded = 0
     for i, ((gb, gst, stored), (wb, wst)) in enumerate(zip(got, want)):
         if wst != 0:
             assert gst == wst, (i, ranges[i], pbs[i], len(syms[i]))
@@ -89,7 +101,9 @@ def test_encode_entropy_batch_random_streams_vs_oracle():
         assert gst == 0 and gb.tobytes() == wb.tobytes(), (i, ranges[i], pbs[i], len(syms[i]))
         n_ok += 1
         n_stored += stored
+        n_low_coded += i >= first_low and not stored
     assert n_ok > 500 and n_stored > 10
+    assert n_low_coded > 40
 
 
 def test_encode_entropy_prefix_and_slab_layout():
@@ -103,7 +117,7 @@ def test_encode_entropy_prefix_and_slab_layout():
 
 
 def test_decode_entropy_vs_oracle_and_roundtrip():
-    """entropy_decoding.hpp:134 — fixed semantics (flags 7) and reference semantics (flags 0)."""
+    """entropy_decoding.hpp:134 — fixed semantics (flags 7) at prob_bits 1..19 and reference semantics (flags 0)."""
     g = gpu_lib.gpu()
     rng = np.random.default_rng(3)
     blobs, offs, caps, exp = [], [], [], []
@@ -135,13 +149,38 @@ def test_decode_entropy_vs_oracle_and_roundtrip():
         exp.append((want, pos + lead + len(enc)))
         pos += lead + len(enc)
     assert lossless > 250
+    # prob_bits 1..7 (k_rans_decode's direct lookup, lut_shift 0), ranges 2..2^prob_bits; drawn after the streams
+    # above so that those stay as they were
+    low = np.random.default_rng(4)
+    first_low = len(exp)
+    for pb in range(1, 8):
+        for rangev in sorted({2, (1 << pb) // 2 + 1, 1 << pb}):
+            for kind in range(6):
+                n = int(low.choice([2, 7, 64, 1000, 20000, 66000]))
+                s = _symbols(low, kind, n, rangev)
+                if len(np.unique(s)) < 2:
+                    s[0] = (int(s[0]) + 1) % rangev
+                enc, st = ol.orc_encode_entropy(s, rangev, pb)
+                assert st == 0
+                want, _, wst = ol.orc_decode_entropy(enc, 0, flags=7, cap=n)
+                assert wst == 0
+                lead = int(low.integers(0, 7))
+                blobs += [np.zeros(lead, np.uint8), enc]
+                offs.append(pos + lead)
+                caps.append(n)
+                exp.append((want if np.array_equal(want, s) else None, pos + lead + len(enc)))
+                pos += lead + len(enc)
     blob = np.concatenate(blobs)
     got = g.decode_entropy_batch(blob, offs, caps, flags=7)
+    low_coded = 0
     for i, ((sym, end, st), (s, e)) in enumerate(zip(got, exp)):
         if s is None:  # garbage table (lossy mode 1): decoded without faulting, or refused as a bad table
             assert st in (0, 3, 6), i  # 6 = HOH_S_BAD_STATE: the final rANS state gives the garbage away
             continue
         assert st == 0 and end == e and np.array_equal(sym, s), i
+        r = g.last_dec_results[i]
+        low_coded += i >= first_low and not r["stored"] and r["prob_bits"] < 8
+    assert low_coded > 30
     # single-call shim, reference semantics: byte_pointer stops at the payload (D8), 4-bit prob_bits (D9)
     checked_ref = 0
     for it in range(40):
